@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N=1: plain python; N>1: torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (outputs of the last timed step)
 
 One "step" = one CCSD iteration with DIIS (dressing -> singles + doubles residual ->
 amplitude update -> DIIS -> energy) on the transcorrelated 3D UEG with 54 electrons in 515
@@ -383,6 +384,26 @@ def dense_ladder_probe(bk, torch, V_abcd, T2, peak, dgemm=None):
         bk.set_blocked(old)
 
 
+DUMP_T2_SAMPLES = 1 << 21          # 16 MiB of T2 values and 16 MiB of their positions
+
+
+def dump_outputs(path, e, T1, T2):
+    """Write what the last timed sweep hands a caller of CCSD.sweep as float64 .npy files under
+    `path`: energy (e_1b, e_dir, e_ex), norms (|T2|, |dT2|), t1 [v, o], and T2 [v, v, o, o] at a
+    fixed, seeded sample of flat positions (t2_sample, positions in t2_sample_index; every position
+    when T2 is smaller than the sample), so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n = T2.numel()
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_T2_SAMPLES), replace=False))
+    idx = torch.from_numpy(pick).to(T2.device)
+    out = {"energy": e[:3], "norms": e[3:5], "t1": T1.cpu().numpy(),
+           "t2_sample": T2[torch.unravel_index(idx, tuple(T2.shape))].cpu().numpy(), "t2_sample_index": pick}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def same_config_leg(cpu, steps_total, torch):
     """The problem the CPU leg timed (TC-UEG 54e in `cpu['n_orb']` plane waves), through the public
     API with HOST buffers on this GPU: numpy Fock / V_pqrs in, `steps_total` CCSD+DIIS sweeps with the
@@ -525,6 +546,8 @@ def run_ours(args):
     bk.enable_trace(False)
     bk.enable_timing(False)
     e_final = e[0] + e[1] + e[2]
+    if args.dump_outputs and rank == 0:     # before the end-to-end sweeps below move the amplitudes on
+        dump_outputs(args.dump_outputs, e, cc._st["T1"], cc._st["T2"])
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -714,10 +737,17 @@ def main():
                          "timed region of a --ladder blocked run")
     ap.add_argument("--dense-abcd", action="store_true",
                     help="store V_abcd in HBM instead of generating it in the ladder kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the energies, T1 and a seeded sample of T2 of the last "
+                         "timed step to DIR/<name>.npy (float64, about 32 MiB)")
     args = ap.parse_args()
     claim_stdout()
     if args.gpus not in CUTOFF_FOR_GPUS:
         raise SystemExit("--gpus must be one of %s" % sorted(CUTOFF_FOR_GPUS))
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        raise SystemExit("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -18,7 +18,24 @@ def pytest_configure(config):
 
 
 def golden(name):
-    return np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
+    """The arrays of tests/golden/<name>.npz.  Where <name>_V.npz exists it holds the integrals
+    V[p,q,r,s], packed by make_golden.py::pack_integrals, and they are rebuilt here exactly."""
+    g = dict(np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False))
+    packed = os.path.join(GOLDEN, name + "_V.npz")
+    if os.path.exists(packed):
+        g["V"] = _unpack_integrals(np.load(packed, allow_pickle=False))
+    return g
+
+
+def _unpack_integrals(packed):
+    """V from its non-zeros with p <= r and q <= s, mirrored by V[p,q,r,s] = V[r,q,p,s] = V[p,s,r,q]."""
+    n = int(packed["n"])
+    keep = np.unpackbits(packed["mask"], count=n ** 4).astype(bool).reshape((n,) * 4)
+    p, q, r, s = np.nonzero(keep)
+    V = np.zeros((n,) * 4)
+    for idx in ((p, q, r, s), (r, q, p, s), (p, s, r, q), (r, s, p, q)):
+        V[idx] = packed["val"]
+    return V
 
 
 @pytest.fixture

@@ -74,10 +74,22 @@ class Tracer:
         return out
 
 
-def molecule(tag, path, is_tc=False, eom_roots=0, delta_e=1e-12, max_iter=200):
+def pack_integrals(V):
+    """V[p,q,r,s] of a real FCIDUMP is exactly invariant under p<->r and under q<->s: keep the
+    non-zeros with p <= r and q <= s.  tests/conftest.py::golden rebuilds V from them exactly."""
+    p, q, r, s = np.indices(V.shape)
+    keep = (p <= r) & (q <= s) & (V != 0)
+    for perm in ((2, 1, 0, 3), (0, 3, 2, 1)):
+        assert np.array_equal(V, V.transpose(perm))
+    return dict(n=V.shape[0], mask=np.packbits(keep.ravel()), val=V[keep])
+
+
+def molecule(tag, path, is_tc=False, eom_roots=0, delta_e=1e-12, max_iter=200, pack_V=False):
     n_elec, nb, e_core, eps, h, V = quiet(fcidump.read, path, is_tc)
     no = n_elec // 2
     out = dict(n_elec=n_elec, e_core=e_core, h=h, V=V, is_tc=is_tc)
+    if pack_V:          # a dense V of 32 orbitals alone would be 3.7 MB compressed
+        save("mol_" + tag + "_V", **pack_integrals(out.pop("V")))
     out["hf_e"] = hf.calc_hf_e(no, e_core, h, V)
     fock = hf.construct_hf_matrix(no, h, V)
     out["fock"] = fock
@@ -119,7 +131,7 @@ def sec_hf_molecule():
     # 32 orbitals, 43 CCSD sweeps: exercises the DIIS-full bookkeeping path
     molecule("HF_augccpvdz",
              os.path.join(TESTDIR, "test_eom_ccsd/FCIDUMP.HF.augccpvdz"),
-             delta_e=1e-8, max_iter=50)
+             delta_e=1e-8, max_iter=50, pack_V=True)
 
 
 def sec_residual_random():
@@ -432,6 +444,8 @@ def sec_ueg_modes():
     # a correlator given without any branch flag: all zeros (the elif chain falls through)
     V = quiet(m.eval_2b_integrals, correlator=m.trunc, sp=0)
     out["big_noflag_absmax"] = np.abs(V).max()
+    save("ueg_modes_branches", **out)       # kept apart: together with the rest it exceeds 1 MB
+    out = {}
     for name, gamma, k_cutoff in (("trunc", None, 1.0), ("coulomb", None, None), ("smooth", None, 1.0),
                                   ("yukawa", None, None), ("yukawa", 0.7, 1.0), ("stg", None, None), ("stg", 1.3, 1.0),
                                   ("yukawa_coulomb", None, None), ("yukawa_coulomb", 1.1, 1.0),

@@ -875,7 +875,7 @@ def test_dots_and_lincomb_beyond_16_vectors(cpu_abi):
 
 
 # --------------------------------------------------------------------------
-# eval_2b_integrals: the remaining branches and every correlator (fixtures: ueg_modes.npz)
+# eval_2b_integrals: the remaining branches and every correlator (fixtures: ueg_modes*.npz)
 # --------------------------------------------------------------------------
 UEG_FLAGS = ["is_rpa_approx", "is_only_hermi_2b", "is_only_non_hermi_2b", "is_exchange_1", "is_exchange_2",
              "is_exchange_3"]
@@ -890,7 +890,7 @@ def test_ueg_remaining_branches_match_reference(cpu_abi, flag):
     """ueg.py:416-423, 440-457, 478-504 with `trunc` at 14e / 57 plane waves against the reference's
     triple loop.  On the CPU emulator a slab of rows, on the GPU the whole tensor."""
     from pymes_b200.model import ueg
-    g = golden("ueg_modes")
+    g = golden("ueg_modes_branches")
     m = ueg.UEG(14, 7, 7, 0.5)
     m.init_single_basis(5.0)
     m.gamma, m.k_cutoff = None, 1.0
