@@ -406,6 +406,41 @@ typedef struct {
 int pmb_gather_expand(const pmb_gather_t *d, pmb_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
+/* Block-diagonal x block-diagonal contraction: two momentum-conserving        */
+/* operands, rows and entries from A, entries and columns from B, all three    */
+/* sorted by group on the host.  Per tile {r0, rn, e0, en, c0, cn}:            */
+/*   C[c_row[r] + c_col[n]] += alpha * sum_{k = e0}^{e0+en-1}                    */
+/*                  A[a_row[r] + a_ent[k]] * B[b_ent[k] + b_col[n]]             */
+/* for r in [r0, r0+rn), n in [c0, c0+cn).  Elements outside every tile are    */
+/* not touched (the caller clears or scales them first).  Every C element      */
+/* belongs to at most one tile; one CTA per tile, FP64 FMA from shared memory, */
+/* fixed summation order, no atomics, no workspace.                            */
+/* ------------------------------------------------------------------------ */
+typedef struct {
+    const double *A;
+    const double *B;
+    double *C;
+    const int64_t *a_row;     /* [rows]    device */
+    const int64_t *a_ent;     /* [entries] device */
+    const int64_t *b_ent;     /* [entries] device */
+    const int64_t *b_col;     /* [columns] device */
+    const int64_t *c_row;     /* [rows]    device */
+    const int64_t *c_col;     /* [columns] device */
+    const int32_t *tiles;     /* [n_tiles][6] device */
+    int32_t n_tiles;
+    int32_t _pad;
+    double alpha;
+} pmb_group_t;
+int pmb_group_contract(const pmb_group_t *d, pmb_stream_t stream);
+
+/* Momentum residue of a strided tensor of rank 1..4:                          */
+/*   out[0] = max |x[i0,..]| over the elements with sum_d key_d[i_d] != 0,       */
+/* key_d = keys + (ext[0] + .. + ext[d-1]) (per-axis signed momentum labels,    */
+/* device), 0 when there is none.  One pass over the tensor; out is device.    */
+int pmb_momentum_residue(int ndim, const int64_t ext[4], const int64_t str[4], const double *x,
+                         const int64_t *keys, double *out, pmb_stream_t stream);
+
+/* ------------------------------------------------------------------------ */
 /* Synthetic non-hermitian integrals (BASELINE.json configs[2]; SURVEY 8(d) C3   */
 /* recipe): out[np][nq][nr][ns] = V[lo[0]+.., lo[1]+.., lo[2]+.., lo[3]+..] with  */
 /*   V[p,q,r,s] = eps * table[ h(seed, c) >> 48 ],                                */

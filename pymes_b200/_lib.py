@@ -70,6 +70,13 @@ class Gather(C.Structure):
                 ("d_jstr", C.c_int64), ("alpha", C.c_double), ("beta", C.c_double)]
 
 
+class Group(C.Structure):
+    _fields_ = [("A", C.c_void_p), ("B", C.c_void_p), ("C", C.c_void_p), ("a_row", C.c_void_p),
+                ("a_ent", C.c_void_p), ("b_ent", C.c_void_p), ("b_col", C.c_void_p), ("c_row", C.c_void_p),
+                ("c_col", C.c_void_p), ("tiles", C.c_void_p), ("n_tiles", C.c_int32), ("_pad", C.c_int32),
+                ("alpha", C.c_double)]
+
+
 _SIGS = {
     "pmb_version": (C.c_int, []),
     "pmb_device_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]),
@@ -109,6 +116,8 @@ _SIGS = {
                                    C.c_void_p, C.c_void_p]),
     "pmb_blocked_contract": (C.c_int, [C.POINTER(Blocked), C.c_void_p]),
     "pmb_gather_expand": (C.c_int, [C.POINTER(Gather), C.c_void_p]),
+    "pmb_group_contract": (C.c_int, [C.POINTER(Group), C.c_void_p]),
+    "pmb_momentum_residue": (C.c_int, [C.c_int, I64x4, I64x4, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pmb_synth_block": (C.c_int, [C.c_int, C.c_ulonglong, C.c_double, C.c_void_p, I32x4, I32x4, C.c_void_p,
                                   C.c_void_p]),
     "pmb_ueg_build_block": (C.c_int, [C.POINTER(Ueg), C.c_void_p, C.c_void_p, C.c_void_p, I32x4, I32x4,

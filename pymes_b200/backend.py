@@ -64,6 +64,10 @@ class GeneratedOperand:
         groups ordered (fastest first) as ``m_ord`` / ``k_ord``."""
         raise NotImplementedError
 
+    def momentum(self):
+        """The operand's :class:`Momentum` selection rule, or None."""
+        return None
+
     def blocked_lists(self):
         """Block-diagonal structure of the operand as the matrix [(axis 0, axis 1), (axis 2, axis 3)]
         for ``pmb_blocked_contract`` (see :func:`_blocked_term`), or None when the source has none."""
@@ -97,8 +101,12 @@ def empty(*shape):
     return torch.empty(shape, dtype=F64, device=device())
 
 
-def zeros(*shape):
-    return torch.zeros(shape, dtype=F64, device=device())
+def zeros(*shape, rule=None):
+    """Zeros; ``rule``: a momentum rule (:class:`Momentum`) to tag them with -- zeros satisfy any."""
+    t = torch.zeros(shape, dtype=F64, device=device())
+    if rule is not None:
+        _set_momentum(t, rule)
+    return t
 
 
 def empty_stacked(shape_a, shape_b):
@@ -578,32 +586,236 @@ def _column_groups(n_sub, ext, bstr, cstr):
     return n0, n1, b1, c1
 
 
+# --------------------------------------------------------------------------
+# momentum tags: which elements of a tensor can be non-zero
+# --------------------------------------------------------------------------
+class Momentum:
+    """Selection rule of a tensor: ``x[i_0, i_1, ..]`` can be non-zero only where
+    ``sum_d sign_d * lin[lo_d + i_d] == 0``, ``lin`` the linearised momentum of every orbital
+    (``model.ueg.momentum_groups``) and one ``(lo, ext, sign)`` per axis.  A stored UEG integral block
+    has signs (+,+,-,-); contractions, linear combinations and index swaps of tensors with such rules
+    have one as well (:func:`contract_terms` derives it), and a tensor from outside gets one only by
+    :func:`adopt_momentum`, which checks it.  A sign 0 leaves its axis unconstrained.  Kept in a
+    normal form (first non-zero sign positive): rules equal up to an overall sign compare equal."""
+
+    __slots__ = ("lin", "lin_key", "axes")
+
+    def __init__(self, lin, axes, lin_key=None):
+        axes = tuple((int(lo), int(n), int(sg)) for lo, n, sg in axes)
+        first = next((sg for _lo, _n, sg in axes if sg), 1)
+        if first < 0:
+            axes = tuple((lo, n, -sg) for lo, n, sg in axes)
+        self.lin = lin
+        self.lin_key = lin_key if lin_key is not None else (lin.tobytes() if lin is not None else None)
+        self.axes = axes
+
+    def __eq__(self, other):
+        return isinstance(other, Momentum) and self.axes == other.axes and self.lin_key == other.lin_key
+
+    def __hash__(self):
+        return hash((self.axes, self.lin_key))
+
+    def with_axes(self, axes):
+        return Momentum(self.lin, axes, self.lin_key)
+
+    def narrow(self, dim, lo, n):
+        axes = list(self.axes)
+        a_lo, _a_n, sg = axes[dim]
+        axes[dim] = (a_lo + int(lo), int(n), sg)
+        return self.with_axes(axes)
+
+    def permute(self, dims):
+        return self.with_axes([self.axes[d] for d in dims])
+
+    def labels(self, d):
+        """Signed momentum labels ``sign * lin[lo:lo+ext]`` of axis ``d`` (int64)."""
+        lo, n, sg = self.axes[d]
+        if sg == 0:
+            return np.zeros(n, dtype=np.int64)
+        return sg * np.asarray(self.lin[lo:lo + n], dtype=np.int64)
+
+
+def _set_momentum(t, key):
+    t._pmb_mom = (key, t._version) if key is not None else None
+
+
+def momentum_of(x):
+    """The live :class:`Momentum` tag of ``x`` (None when there is none, or when the tensor was
+    edited in place after it was tagged: the tag records the tensor's version counter)."""
+    if isinstance(x, GeneratedOperand):
+        return x.momentum()
+    if not isinstance(x, torch.Tensor):
+        return None
+    tag = getattr(x, "_pmb_mom", None)
+    if tag is not None and tag[1] == x._version:
+        return tag[0]
+    # a view of a tensor whose rule is live (written through a sibling view since it was made)
+    link = getattr(x, "_pmb_parent", None)
+    if link is not None:
+        pk = momentum_of(link[0])
+        if pk is not None:
+            return pk.narrow(*link[1:])
+    return None
+
+
+def ones(n):
+    """A vector of ones; it satisfies the rule without constraint (sign 0)."""
+    t = torch.ones(n, dtype=F64, device=device())
+    _set_momentum(t, Momentum(None, [(0, n, 0)]))
+    return t
+
+
+def adopt_momentum(t, key, host=None):
+    """Tag ``t`` (a tensor that enters from outside) with the rule ``key`` if and only if every
+    element the rule forbids is exactly zero (``pmb_momentum_residue``: one pass over the tensor).
+    ``host``: the same values as a numpy array the caller holds anyway (e.g. the Fock matrix); they
+    are checked there instead.  Returns True when it was tagged."""
+    if key is None or not isinstance(t, torch.Tensor) or t.dim() != len(key.axes) or not 1 <= t.dim() <= 4:
+        return False
+    if any(int(n) != a[1] for n, a in zip(t.shape, key.axes)):
+        raise ValueError("momentum rule %s does not fit a tensor of shape %s" % (key.axes, tuple(t.shape)))
+    if host is not None:
+        host = np.asarray(host)
+        if host.shape != tuple(t.shape):
+            raise ValueError("host copy of shape %s for a tensor of shape %s" % (host.shape, tuple(t.shape)))
+        total = np.zeros((), dtype=np.int64)
+        for d in range(t.dim()):
+            total = np.add.outer(total, key.labels(d))
+        ok = not np.any(host[total != 0] != 0)           # NaN != 0: not adopted
+        _set_momentum(t, key if ok else None)
+        return ok
+    labels = torch.from_numpy(np.concatenate([key.labels(d) for d in range(t.dim())])).to(device())
+    res = zeros(1)
+    _lib.check(_lib.load().pmb_momentum_residue(t.dim(), _lib.I64x4(*_pad4r(t.shape, 1)),
+                                                 _lib.I64x4(*_pad4r(t.stride(), 0)), _ptr(t), _ptr(labels),
+                                                 _ptr(res), _stream()), "pmb_momentum_residue")
+    ok = float(res.item()) == 0.0
+    _set_momentum(t, key if ok else None)
+    return ok
+
+
+def drop_momentum(t):
+    """Remove the momentum tag of ``t`` (always safe: the tensor then takes the dense paths)."""
+    if isinstance(t, torch.Tensor):
+        _set_momentum(t, None)
+
+
+def _pad4r(vals, fill):
+    vals = [int(v) for v in vals]
+    return vals + [fill] * (4 - len(vals))
+
+
+def _chain(out):
+    """``[(parent, dim, lo, n, parent's live tag)]`` up the :func:`narrow` chain of ``out``, read
+    BEFORE a write into it."""
+    links, t = [], out
+    while True:
+        link = getattr(t, "_pmb_parent", None)
+        if link is None:
+            return links
+        p, dim, lo, n = link
+        links.append((p, dim, lo, n, momentum_of(p)))
+        t = p
+
+
+def _written(out, key, chain):
+    """A backend kernel has written ``out``: its storage changed behind torch's back, so the version
+    counter it shares with its base and every other view is bumped (their tags die), then ``out``
+    gets ``key``.  A :func:`narrow` parent whose rule, restricted to the view, is ``key`` keeps its
+    tag: the write stayed inside its selection rule."""
+    torch.autograd.graph.increment_version(out)
+    _set_momentum(out, key)
+    child = key
+    for p, dim, lo, n, pk in chain:
+        if child is None or pk is None or pk.narrow(dim, lo, n) != child:
+            break
+        _set_momentum(p, pk)
+        child = pk
+
+
+def _term_keys(out_sub, sa, ka, sb, kb):
+    """The rules the product ``einsum(sa, sb -> out_sub)`` of operands with rules ``ka`` / ``kb``
+    satisfies: with one sign sigma for the whole term, every summed axis must cancel
+    (``sign_a + sigma * sign_b == 0`` over the same orbitals); the output axes then carry the signs
+    of A and sigma times those of B.  Both sigmas when nothing constrains it (outer products)."""
+    if ka.lin_key is not None and kb.lin_key is not None and ka.lin_key != kb.lin_key:
+        return set()
+    lin, lin_key = (ka.lin, ka.lin_key) if ka.lin_key is not None else (kb.lin, kb.lin_key)
+    xa, xb = dict(zip(sa, ka.axes)), dict(zip(sb, kb.axes))
+    sigmas = {1, -1}
+    for ch in sa:
+        if ch not in sb:
+            if ch not in out_sub:
+                return set()
+            continue
+        if ch in out_sub:
+            return set()
+        (la, na, ga), (lb, nb, gb) = xa[ch], xb[ch]
+        if ga == 0 and gb == 0:
+            continue
+        if (la, na) != (lb, nb) or abs(ga) != abs(gb):
+            return set()
+        sigmas &= {-1 if ga == gb else 1}
+    if any(ch not in sa and ch not in out_sub for ch in sb) or any(ch not in xa and ch not in xb for ch in out_sub):
+        return set()
+    return {Momentum(lin, [xa[ch] if ch in xa else (xb[ch][0], xb[ch][1], sg * xb[ch][2]) for ch in out_sub],
+                     lin_key) for sg in sigmas}
+
+
+def _derive(out_sub, terms, old, accumulate):
+    """The rule of ``out = beta*out + sum of terms``: one that every term satisfies (and, when the
+    output accumulates, the one it already has); None when there is none."""
+    if accumulate and old is None:
+        return None
+    cands = None
+    for _alpha, sa, A, sb, B in terms:
+        ka, kb = momentum_of(A), momentum_of(B)
+        if ka is None or kb is None or len(ka.axes) != len(sa) or len(kb.axes) != len(sb):
+            return None
+        c = _term_keys(out_sub, sa, ka, sb, kb)
+        cands = c if cands is None else cands & c
+        if not cands:
+            return None
+    if old is not None:
+        return old if old in cands else None
+    return min(cands, key=lambda k: k.axes)
+
+
 def tag_geom(t, geom):
     """Attach the (p,q,r,s) geometry of a stored integral block to its tensor (see
-    ``model.ueg.MomentumGeom``); returns the tensor."""
-    t._pmb_geom = geom
+    ``model.ueg.MomentumGeom``) together with its momentum rule; returns the tensor."""
+    t._pmb_geom = (geom, t._version)
+    _set_momentum(t, geom.momentum())
     return t
 
 
 def geom_of(t):
-    return getattr(t, "_pmb_geom", None) if isinstance(t, torch.Tensor) else None
+    """The live geometry tag of a stored integral block (None after an in-place edit)."""
+    tag = getattr(t, "_pmb_geom", None) if isinstance(t, torch.Tensor) else None
+    if tag is None or tag[1] != t._version:
+        return None
+    return tag[0]
 
 
 def narrow(t, dim, lo, n):
-    """``t.narrow(dim, lo, n)`` that keeps the geometry tag of a stored integral block."""
+    """``t.narrow(dim, lo, n)`` that keeps the tags of ``t``, restricted to the view."""
     out = t.narrow(dim, lo, n)
     g = geom_of(t)
     if g is not None:
-        out._pmb_geom = g.narrow(dim, lo, n)
+        out._pmb_geom = (g.narrow(dim, lo, n), out._version)
+    k = momentum_of(t)
+    if k is not None:
+        _set_momentum(out, k.narrow(dim, lo, n))
+    out._pmb_parent = (t, int(dim), int(lo), int(n))
     return out
 
 
-def copy_tagged(src):
-    """A copy of a stored integral block that IS the block (same values): keeps the tag."""
-    out = copy(src)
-    g = geom_of(src)
-    if g is not None:
-        out._pmb_geom = g
+def permute(t, dims):
+    """``t.permute(dims)`` that keeps the momentum tag of ``t``."""
+    out = t.permute(*dims)
+    k = momentum_of(t)
+    if k is not None:
+        _set_momentum(out, k.permute(dims))
     return out
 
 
@@ -679,8 +891,13 @@ def _run_blocked(out_sub, term, out, beta):
     if offs is None:
         offs = (up(L["row_i0"] * key[0] + L["row_i1"] * key[1]), up(L["ent_j0"] * key[2] + L["ent_j1"] * key[3]))
         L["offsets"][key] = offs
-    if beta == 0.0 and not L["rows_covered"]:
-        out.zero_()              # rows outside every group are part of the result: zero
+    if beta != 1.0 and not L["rows_covered"]:
+        # rows outside every group are part of the result: zero, or scaled by beta
+        if beta == 0.0:
+            out.zero_()
+        else:
+            axpby(beta, out, 0.0, out)
+        beta = 1.0
     d = _lib.Blocked()
     d.A, d.B, d.C = values.data_ptr(), B.data_ptr(), out.data_ptr()
     d.a_moff, d.a_koff = a_moff.data_ptr(), a_koff.data_ptr()
@@ -775,36 +992,165 @@ def _try_gather(out_sub, terms, out, beta):
     return out
 
 
+def _group_term(out_sub, term):
+    """``(alpha, sa, A, sb, B, sigma)`` if this term can go to ``pmb_group_contract``: both operands
+    stored tensors with a live momentum rule, and the split 2 | 2 | 2 (two output indices from A,
+    two summed, two output indices from B) with the summed axes cancelling under one sign sigma.
+    Else None."""
+    if not _BLOCKED[0]:
+        return None
+    alpha, sa, A, sb, B = term
+    if not (isinstance(A, torch.Tensor) and isinstance(B, torch.Tensor)):
+        return None
+    if len(sa) != 4 or len(sb) != 4 or len(out_sub) != 4 or A.dim() != 4 or B.dim() != 4:
+        return None
+    if len(set(sa)) != 4 or len(set(sb)) != 4 or len(set(out_sub)) != 4:
+        return None
+    ka, kb = momentum_of(A), momentum_of(B)
+    if ka is None or kb is None or not _term_keys(out_sub, sa, ka, sb, kb):
+        return None
+    rows = [ch for ch in sa if ch in out_sub]
+    cols = [ch for ch in sb if ch in out_sub]
+    ents = [ch for ch in sa if ch not in out_sub]
+    if len(rows) != 2 or len(cols) != 2 or sorted(ents) != sorted(ch for ch in sb if ch not in out_sub):
+        return None
+    ga, gb = ka.axes[sa.index(ents[0])][2], kb.axes[sb.index(ents[0])][2]
+    if ga == 0 or gb == 0:
+        return None
+    return float(alpha), sa, A, sb, B, (-1 if ga == gb else 1)
+
+
+_GROUP_CACHE = {}
+GROUP_TILE = 32          # rows / columns per tile of pmb_group_contract (its GT)
+
+
+def _sorted_side(labels):
+    """Stable order of a side's flat positions by label, its distinct labels, first positions, counts."""
+    order = np.argsort(labels, kind="stable")
+    keys, first, cnt = np.unique(labels[order], return_index=True, return_counts=True)
+    return order, keys, first, cnt
+
+
+def _group_plan(out_sub, g, out):
+    """Device lists and tiles of one group term, cached by value: the three sides' momentum labels
+    and the strides of A, B and C (intermediates are new tensors every sweep and hit the cache)."""
+    _alpha, sa, A, sb, B, sigma = g
+    ka, kb = momentum_of(A), momentum_of(B)
+    rows = [sa.index(ch) for ch in sa if ch in out_sub]
+    ents = [sa.index(ch) for ch in sa if ch not in out_sub]
+    cols = [sb.index(ch) for ch in sb if ch in out_sub]
+    b_ents = [sb.index(sa[d]) for d in ents]
+    cstr = dict(zip(out_sub, out.stride()))
+    key = (ka.lin_key, tuple(ka.axes[d] for d in rows + ents), tuple(kb.axes[d] for d in cols), sigma,
+           tuple(A.stride(d) for d in rows + ents), tuple(B.stride(d) for d in b_ents + cols),
+           tuple(cstr[sa[d]] for d in rows), tuple(cstr[sb[d]] for d in cols), str(out.device))
+    plan = _GROUP_CACHE.get(key)
+    if plan is not None:
+        return plan
+    outer = lambda x, y: (x[:, None] + y[None, :]).reshape(-1)
+    r_lab = outer(ka.labels(rows[0]), ka.labels(rows[1]))
+    e_lab = -outer(ka.labels(ents[0]), ka.labels(ents[1]))
+    c_lab = -sigma * outer(kb.labels(cols[0]), kb.labels(cols[1]))
+    r_ord, r_key, r_first, r_cnt = _sorted_side(r_lab)
+    e_ord, e_key, e_first, e_cnt = _sorted_side(e_lab)
+    c_ord, c_key, c_first, c_cnt = _sorted_side(c_lab)
+    common = np.intersect1d(np.intersect1d(r_key, e_key, assume_unique=True), c_key, assume_unique=True)
+    ri, ei, ci = (np.searchsorted(k, common) for k in (r_key, e_key, c_key))
+    tiles = []
+    for g0, (r0, rn, e0, en, c0, cn) in enumerate(zip(r_first[ri], r_cnt[ri], e_first[ei], e_cnt[ei],
+                                                     c_first[ci], c_cnt[ci])):
+        for rt in range(0, int(rn), GROUP_TILE):
+            for ct_ in range(0, int(cn), GROUP_TILE):
+                tiles.append((r0 + rt, min(GROUP_TILE, rn - rt), e0, en, c0 + ct_, min(GROUP_TILE, cn - ct_)))
+    tiles = np.asarray(tiles, dtype=np.int32).reshape(-1, 6)
+    n1 = lambda d, t: int(t.shape[d])
+    dev = out.device
+    up = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64)).to(dev)
+    ra, rb_ = r_ord // n1(rows[1], A), r_ord % n1(rows[1], A)
+    ea, eb = e_ord // n1(ents[1], A), e_ord % n1(ents[1], A)
+    ca, cb = c_ord // n1(cols[1], B), c_ord % n1(cols[1], B)
+    plan = dict(
+        a_row=up(ra * A.stride(rows[0]) + rb_ * A.stride(rows[1])),
+        a_ent=up(ea * A.stride(ents[0]) + eb * A.stride(ents[1])),
+        b_ent=up(ea * B.stride(b_ents[0]) + eb * B.stride(b_ents[1])),
+        b_col=up(ca * B.stride(cols[0]) + cb * B.stride(cols[1])),
+        c_row=up(ra * cstr[sa[rows[0]]] + rb_ * cstr[sa[rows[1]]]),
+        c_col=up(ca * cstr[sb[cols[0]]] + cb * cstr[sb[cols[1]]]),
+        tiles=torch.from_numpy(np.ascontiguousarray(tiles)).to(dev), n_tiles=len(tiles),
+        flops=2.0 * float((r_cnt[ri] * e_cnt[ei] * c_cnt[ci]).sum()))
+    _GROUP_CACHE[key] = plan
+    return plan
+
+
+def _run_group(out_sub, g, out, beta):
+    """One term through ``pmb_group_contract``.  Elements outside every group get no product: they
+    are cleared (beta = 0) or scaled (beta != 1) here, before the kernel accumulates."""
+    alpha, sa, A, sb, B, _sigma = g
+    plan = _group_plan(out_sub, g, out)
+    if beta == 0.0:
+        out.zero_()
+    elif beta != 1.0:
+        axpby(beta, out, 0.0, out)
+    d = _lib.Group()
+    d.A, d.B, d.C = A.data_ptr(), B.data_ptr(), out.data_ptr()
+    d.a_row, d.a_ent, d.b_ent = plan["a_row"].data_ptr(), plan["a_ent"].data_ptr(), plan["b_ent"].data_ptr()
+    d.b_col, d.c_row, d.c_col = plan["b_col"].data_ptr(), plan["c_row"].data_ptr(), plan["c_col"].data_ptr()
+    d.tiles, d.n_tiles, d.alpha = plan["tiles"].data_ptr(), int(plan["n_tiles"]), alpha
+    trace = _timing["trace"]
+    if trace is not None:
+        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        t0.record(torch.cuda.current_stream())
+    rc = _lib.load().pmb_group_contract(C.byref(d), _stream())
+    if trace is not None:
+        t1.record(torch.cuda.current_stream())
+        trace.append(("%s,%s->%s [momentum-blocked]" % (sa, sb, out_sub), plan["flops"], t0, t1))
+    _lib.check(rc, "pmb_group_contract")
+
+
 def _try_blocked(out_sub, terms, out, beta):
-    """Terms with a momentum-structured operand (``_blocked_term``: a generated integral block or a
-    stored one with a geometry tag) are
-    evaluated by ``pmb_blocked_contract`` on the diagonal blocks only; the other terms of the same
-    call (e.g. the hole-hole ladder next to the particle-particle one, ccd.py:185-187) keep the
-    dense kernel.  Returns the result, or None when no term qualifies."""
-    picked = [(i, _blocked_term(out_sub, t)) for i, t in enumerate(terms)]
-    picked = [(i, t) for i, t in picked if t is not None]
+    """Terms with momentum structure are evaluated on their diagonal blocks only: both operands
+    with a live momentum rule and a 2 | 2 | 2 split by ``pmb_group_contract`` (``_group_term``), a
+    stored or generated integral block times a dense operand by ``pmb_blocked_contract``
+    (``_blocked_term``).  The other terms of the same call (e.g. the hole-hole ladder next to the
+    particle-particle one, ccd.py:185-187) keep the dense kernel.  Returns the result, or None when
+    no term qualifies."""
+    picked = []
+    for i, t in enumerate(terms):
+        g = _group_term(out_sub, t)
+        if g is not None:
+            picked.append((i, "group", g))
+            continue
+        b = _blocked_term(out_sub, t)
+        if b is not None:
+            picked.append((i, "blocked", b))
     if not picked:
         return None
+    _alpha, sa, A, sb, B = picked[0][2][:5]
+    ext = dict(zip(sb, (int(n) for n in B.shape)))
+    ext.update(zip(sa, (int(n) for n in A.shape)))
+    shape = tuple(ext[ch] for ch in out_sub)
     if out is None:
         if beta != 0.0:
             raise ValueError("beta != 0 needs an output tensor")
-        alpha, sa, A, sb, B, m_axes, _k = picked[0][1]
-        ext = dict(zip(sb, B.shape))
-        ext.update((sa[i], A.shape[i]) for i in m_axes)
-        out = empty(*[int(ext[ch]) for ch in out_sub])
+        out = empty(*shape)
+    elif tuple(out.shape) != shape:
+        raise ValueError("output shape %s != %s" % (tuple(out.shape), shape))
     elif out.device != device():
         raise RuntimeError("pymes_b200: output tensor lives on %s, the kernels write to %s "
                            "(there is no CPU fallback)" % (out.device, device()))
     done = set()
-    rest = [t for i, t in enumerate(terms) if i not in {j for j, _ in picked}]
+    rest = [t for i, t in enumerate(terms) if i not in {j for j, _k, _t in picked}]
     if rest:
         contract_terms(out_sub, rest, out=out, beta=beta)
         beta = 1.0
-    for i, t in picked:
-        if _run_blocked(out_sub, t, out, beta):
-            done.add(i)
-            beta = 1.0
-    left = [terms[i] for i, _ in picked if i not in done]
+    for i, kind, t in picked:
+        if kind == "group":
+            _run_group(out_sub, t, out, beta)
+        elif not _run_blocked(out_sub, t, out, beta):
+            continue
+        done.add(i)
+        beta = 1.0
+    left = [terms[i] for i, _k, _t in picked if i not in done]
     if left:
         old = set_blocked(False)
         try:
@@ -821,7 +1167,19 @@ def contract_terms(out_sub, terms, out=None, beta=0.0):
     output indices between their two operands in the same way (operands are
     swapped automatically when needed); contracted indices may differ per term.
     One kernel launch accumulates every term in registers.
+
+    The result carries the momentum rule every term derives from its operands' rules (and, when
+    ``beta != 0``, the one ``out`` already had); otherwise none.
     """
+    accumulate = out is not None and beta != 0.0
+    chain = _chain(out) if out is not None else []
+    key = _derive(out_sub, terms, momentum_of(out) if accumulate else None, accumulate)
+    out = _contract_terms(out_sub, terms, out, beta)
+    _written(out, key, chain)
+    return out
+
+
+def _contract_terms(out_sub, terms, out, beta):
     lib = _lib.load()
     if out is not None and out.device != device():
         raise RuntimeError("pymes_b200: output tensor lives on %s, the kernels write to %s "
@@ -883,16 +1241,25 @@ def axpby(alpha, src, beta=0.0, out=None):
         out = empty(*src.shape)
     if tuple(out.shape) != tuple(src.shape):
         raise ValueError("shape mismatch")
+    key, chain = momentum_of(src), _chain(out)
+    if beta != 0.0 and momentum_of(out) != key:
+        key = None
     ext = _lib.I64x4(*_pad4(src.shape, 1))
     si = _lib.I64x4(*_pad4(src.stride(), 0))
     so = _lib.I64x4(*_pad4(out.stride(), 0))
     _lib.check(lib.pmb_axpby4(ext, float(alpha), _ptr(src), si, float(beta), _ptr(out), so, _stream()),
                "pmb_axpby4")
+    _written(out, key, chain)
     return out
 
 
 def copy(src):
-    return axpby(1.0, src)
+    """A copy keeps the tags of its source (a copy of a stored integral block IS the block)."""
+    out = axpby(1.0, src)
+    g = geom_of(src)
+    if g is not None:
+        out._pmb_geom = (g, out._version)
+    return out
 
 
 def mp2_amplitudes(eps_i, eps_a, shift, V_abij, rows=None):
@@ -904,6 +1271,7 @@ def mp2_amplitudes(eps_i, eps_a, shift, V_abij, rows=None):
     _lib.check(lib.pmb_mp2_amplitudes(no, nv, a_lo, na, _ptr(eps_i), _ptr(eps_a), float(shift), _ptr(V_abij),
                                       _lib.I64x4(*V_abij.stride()), _ptr(T2), _stream()),
                "pmb_mp2_amplitudes")
+    _written(T2, momentum_of(V_abij), [])        # the denominators are diagonal: same rule
     return T2
 
 
@@ -918,11 +1286,14 @@ def update_doubles(eps_i, eps_a, shift, delta, R, T2, scal, rows=None, product_d
     no, nv = eps_i.numel(), eps_a.numel()
     a_lo, na = rows if rows is not None else (0, nv)
     dT = torch.empty_like(T2)
+    kR, kT, chain = momentum_of(R), momentum_of(T2), _chain(T2)
     ws = scratch().reduce_ws()
     _lib.check(lib.pmb_update_doubles(no, nv, a_lo, na, _ptr(eps_i), _ptr(eps_a), float(shift), float(delta),
                                       int(bool(product_denominator)), _ptr(R), _ptr(dT), _ptr(T2), _ptr(scal),
                                       _ptr(ws), ws.numel() * 8,
                                       _stream()), "pmb_update_doubles")
+    _written(dT, kR, [])
+    _written(T2, kT if kT == kR else None, chain)
     return dT
 
 
@@ -930,8 +1301,11 @@ def update_singles(eps_i, eps_a, shift, delta, R1, T1):
     lib = _lib.load()
     no, nv = eps_i.numel(), eps_a.numel()
     dT1 = torch.empty_like(T1)
+    kR, kT, chain = momentum_of(R1), momentum_of(T1), _chain(T1)
     _lib.check(lib.pmb_update_singles(no, nv, _ptr(eps_i), _ptr(eps_a), float(shift), float(delta), _ptr(R1),
                                       _ptr(dT1), _ptr(T1), _stream()), "pmb_update_singles")
+    _written(dT1, kR, [])
+    _written(T1, kT if kT == kR else None, chain)
     return dT1
 
 
@@ -952,7 +1326,10 @@ def tilde(T2, swap_ij=False):
     lib = _lib.load()
     nv, no = T2.shape[0], T2.shape[2]
     Tt = torch.empty_like(T2)
+    k = momentum_of(T2)
     _lib.check(lib.pmb_tilde(no, nv, _ptr(T2), _ptr(Tt), int(swap_ij), _stream()), "pmb_tilde")
+    # 2 T - T with two indices swapped: the rule survives when the swap leaves it unchanged
+    _written(Tt, k if k is not None and k.permute((0, 1, 3, 2) if swap_ij else (1, 0, 2, 3)) == k else None, [])
     return Tt
 
 
@@ -962,7 +1339,11 @@ def sym_baji(Ex, R=None, accumulate=True):
     nv, no = Ex.shape[0], Ex.shape[2]
     if R is None:
         R, accumulate = torch.empty_like(Ex), False
+    k, chain = momentum_of(Ex), _chain(R)
+    if k is not None and (k.permute((1, 0, 3, 2)) != k or (accumulate and momentum_of(R) != k)):
+        k = None
     _lib.check(lib.pmb_sym_baji(no, nv, _ptr(Ex), _ptr(R), int(accumulate), _stream()), "pmb_sym_baji")
+    _written(R, k, chain)
     return R
 
 
@@ -997,6 +1378,8 @@ def lincomb(coefs, xs, out=None, beta=0.0):
             raise ValueError("lincomb needs contiguous tensors")
     if out is None:
         out = torch.empty_like(xs[0])
+    keys = {momentum_of(t) for t in xs} | ({momentum_of(out)} if beta != 0.0 else set())
+    key, chain = (keys.pop() if len(keys) == 1 else None), _chain(out)
     done = 0
     while done < len(xs):
         chunk = xs[done:done + 16]
@@ -1004,6 +1387,7 @@ def lincomb(coefs, xs, out=None, beta=0.0):
         _lib.check(lib.pmb_lincomb(len(chunk), c, _ptr_array(chunk), out.numel(),
                                    float(beta) if done == 0 else 1.0, _ptr(out), _stream()), "pmb_lincomb")
         done += len(chunk)
+    _written(out, key, chain)
     return out
 
 
@@ -1046,7 +1430,9 @@ def bdot(spec, A, B, out=None, alpha=1.0, beta=0.0):
     _fill(d.r_ext, [ext[ch] for ch in rord])
     _fill(d.a_rstr, [astr[ch] for ch in rord])
     _fill(d.b_rstr, [bstr[ch] for ch in rord])
+    chain = _chain(out)
     _lib.check(lib.pmb_bdot(C.byref(d), _stream()), "pmb_bdot")
+    _written(out, None, chain)
     return out
 
 
@@ -1069,8 +1455,19 @@ def diag_view(t, sub, out_sub):
             raise ValueError("repeated index %s with different extents" % ch)
     if set(out_sub) != set(sub):
         raise ValueError("diag_view keeps every index: %s -> %s" % (sub, out_sub))
-    return torch.as_strided(t, [sizes[ch] for ch in out_sub], [strides[ch] for ch in out_sub],
+    view = torch.as_strided(t, [sizes[ch] for ch in out_sub], [strides[ch] for ch in out_sub],
                             t.storage_offset())
+    k = momentum_of(t)
+    if k is not None:
+        # a repeated index carries the sum of its axes' signs (the axes must cover the same orbitals)
+        axes = {}
+        for ch, (lo, n, sg) in zip(sub, k.axes):
+            lo0, n0, sg0 = axes.get(ch, (lo, n, 0))
+            if (lo0, n0) != (lo, n):
+                return view
+            axes[ch] = (lo, n, sg0 + sg)
+        _set_momentum(view, k.with_axes([axes[ch] for ch in out_sub]))
+    return view
 
 
 def add_broadcast(alpha, src, src_sub, out, out_sub):
@@ -1082,7 +1479,9 @@ def add_broadcast(alpha, src, src_sub, out, out_sub):
     ext = _lib.I64x4(*_pad4(out.shape, 1))
     si = _lib.I64x4(*_pad4([sstr.get(ch, 0) for ch in out_sub], 0))
     so = _lib.I64x4(*_pad4(out.stride(), 0))
+    chain = _chain(out)
     _lib.check(lib.pmb_axpby4(ext, float(alpha), _ptr(src), si, 1.0, _ptr(out), so, _stream()), "pmb_axpby4")
+    _written(out, None, chain)
     return out
 
 
@@ -1129,7 +1528,7 @@ def einsum(spec, *ops, out=None, alpha=1.0, beta=0.0):
             ext[ch] = int(n)
     if len(items) == 1:
         s, t = items[0]
-        src = t.permute(*[s.index(ch) for ch in so])
+        src = permute(t, [s.index(ch) for ch in so])
         return axpby(alpha, src, beta, out)
     while len(items) > 2:
         best = None

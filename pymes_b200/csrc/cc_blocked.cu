@@ -276,3 +276,153 @@ extern "C" int pmb_gather_expand(const pmb_gather_t *d, pmb_stream_t stream) {
     count_launch();
     return cuda_status();
 }
+
+// ---------------------------------------------------------------------------
+// pmb_group_contract: both operands momentum-conserving (amplitudes, ring intermediates).
+//
+// A ring product such as "kaic,cbkj->abij" (ccd.py:233) of two tensors that are each non-zero only
+// where their signed momenta sum to zero is block diagonal in ALL three index pairs at once: rows
+// (a,i), entries (k,c) and columns (b,j) with the same group key g meet only each other.  At 54
+// electrons / 515 plane waves that is 1140 groups of at most 27 x 27 x 27 instead of one
+// 13176 x 13176 x 13176 product.  The host sorts the three lists by group and cuts each group into
+// tiles of <= 32 rows x 32 columns; one CTA owns a tile, gathers 32-entry slabs of A and B into
+// shared memory and accumulates with FP64 FMA (2 x 2 outputs per thread).  The work per product is
+// a few 10^7 flop, so the tensor cores would buy nothing here; what matters is that no zero is
+// read.  Each C element belongs to one tile: deterministic, no atomics.
+// ---------------------------------------------------------------------------
+namespace pmb {
+namespace {
+
+constexpr int GT = 32, GK = 32, GNT = 256;
+
+__global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_group_t p) {
+    __shared__ double As[GK][GT + 1];
+    __shared__ double Bs[GK][GT + 1];
+    __shared__ long long s_ar[GT], s_cr[GT], s_bc[GT], s_cc[GT];
+    const int *tl = p.tiles + 6 * (size_t)blockIdx.x;
+    const int r0 = tl[0], rn = tl[1], e0 = tl[2], en = tl[3], c0 = tl[4], cn = tl[5];
+    const int tid = threadIdx.x;
+    if (tid < GT) {
+        const bool ok = tid < rn;
+        s_ar[tid] = ok ? p.a_row[r0 + tid] : 0;
+        s_cr[tid] = ok ? p.c_row[r0 + tid] : 0;
+    } else if (tid < 2 * GT) {
+        const int j = tid - GT;
+        const bool ok = j < cn;
+        s_bc[j] = ok ? p.b_col[c0 + j] : 0;
+        s_cc[j] = ok ? p.c_col[c0 + j] : 0;
+    }
+    const int tx = tid % 16, ty = tid / 16;       // columns tx, tx+16; rows ty, ty+16
+    double acc[2][2] = {{0.0, 0.0}, {0.0, 0.0}};
+    for (int kc = 0; kc < en; kc += GK) {
+        __syncthreads();                          // offsets staged / previous slab consumed
+        for (int idx = tid; idx < GK * GT; idx += GNT) {
+            const int k = idx / GT, m = idx % GT;
+            const bool kok = kc + k < en;
+            const long long ae = kok ? __ldg(p.a_ent + e0 + kc + k) : 0;
+            const long long be = kok ? __ldg(p.b_ent + e0 + kc + k) : 0;
+            As[k][m] = (kok && m < rn) ? __ldg(p.A + s_ar[m] + ae) : 0.0;
+            Bs[k][m] = (kok && m < cn) ? __ldg(p.B + be + s_bc[m]) : 0.0;
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int k = 0; k < GK; ++k) {
+            const double a0 = As[k][ty], a1 = As[k][ty + 16];
+            const double b0 = Bs[k][tx], b1 = Bs[k][tx + 16];
+            acc[0][0] = fma(a0, b0, acc[0][0]);
+            acc[0][1] = fma(a0, b1, acc[0][1]);
+            acc[1][0] = fma(a1, b0, acc[1][0]);
+            acc[1][1] = fma(a1, b1, acc[1][1]);
+        }
+    }
+    if (en <= 0) __syncthreads();                 // the offsets above are visible
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+        const int m = ty + 16 * i;
+        if (m >= rn) continue;
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            const int n = tx + 16 * j;
+            if (n >= cn) continue;
+            double *c = p.C + s_cr[m] + s_cc[n];
+            *c += p.alpha * acc[i][j];
+        }
+    }
+}
+
+// One pass over a strided tensor: max |x| where the signed momenta of its indices do not cancel.
+// Non-negative doubles order like their bit patterns, so the maximum is an integer atomicMax.
+struct Residue {
+    long long ext[4], str[4], koff[4];   // koff < 0: the axis is absent (extent 1, key 0)
+};
+
+__device__ __forceinline__ long long axis_key(const long long *keys, long long koff, long long i) {
+    return koff < 0 ? 0 : __ldg(keys + koff + i);
+}
+
+__global__ void __launch_bounds__(256) residue_kernel(const __grid_constant__ Residue s, const double *x,
+                                                      const long long *keys, unsigned long long *out) {
+    __shared__ unsigned long long red[256];
+    const long long total = s.ext[0] * s.ext[1] * s.ext[2] * s.ext[3];
+    unsigned long long best = 0;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total;
+         e += (long long)gridDim.x * blockDim.x) {
+        long long q = e;
+        const long long i3 = q % s.ext[3]; q /= s.ext[3];
+        const long long i2 = q % s.ext[2]; q /= s.ext[2];
+        const long long i1 = q % s.ext[1];
+        const long long i0 = q / s.ext[1];
+        const long long sum = axis_key(keys, s.koff[0], i0) + axis_key(keys, s.koff[1], i1) +
+                              axis_key(keys, s.koff[2], i2) + axis_key(keys, s.koff[3], i3);
+        if (sum == 0) continue;
+        const double v = fabs(x[i0 * s.str[0] + i1 * s.str[1] + i2 * s.str[2] + i3 * s.str[3]]);
+        const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+        best = b > best ? b : best;
+    }
+    red[threadIdx.x] = best;
+    __syncthreads();
+    for (int w = 128; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w && red[threadIdx.x + w] > red[threadIdx.x]) red[threadIdx.x] = red[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0 && red[0] != 0) atomicMax(out, red[0]);
+}
+
+}  // namespace
+}  // namespace pmb
+
+extern "C" int pmb_group_contract(const pmb_group_t *d, pmb_stream_t stream) {
+    if (!d || d->n_tiles < 0) return PMB_E_BADARG;
+    if (d->n_tiles == 0) return 0;
+    if (!d->A || !d->B || !d->C || !d->a_row || !d->a_ent || !d->b_ent || !d->b_col || !d->c_row ||
+        !d->c_col || !d->tiles)
+        return PMB_E_BADARG;
+    group_kernel<<<(unsigned)d->n_tiles, GNT, 0, (cudaStream_t)stream>>>(*d);
+    count_launch();
+    return cuda_status();
+}
+
+extern "C" int pmb_momentum_residue(int ndim, const int64_t ext[4], const int64_t str[4], const double *x,
+                                    const int64_t *keys, double *out, pmb_stream_t stream) {
+    if (ndim < 1 || ndim > 4 || !ext || !str || !x || !keys || !out) return PMB_E_BADARG;
+    // right-align the axes: missing leading axes have extent 1 and no key
+    Residue s;
+    long long total = 1, koff = 0;
+    for (int d = 0; d < 4; ++d) {
+        const int src = d - (4 - ndim);
+        s.ext[d] = src >= 0 ? ext[src] : 1;
+        s.str[d] = src >= 0 ? str[src] : 0;
+        s.koff[d] = src >= 0 ? koff : -1;
+        if (s.ext[d] < 1) return PMB_E_BADARG;
+        if (src >= 0) koff += ext[src];
+        total *= s.ext[d];
+    }
+    cudaError_t e = cudaMemsetAsync(out, 0, sizeof(double), (cudaStream_t)stream);
+    if (e != cudaSuccess) return (int)e;
+    long long blocks = (total + 255) / 256;
+    if (blocks > 8LL * kSmCount) blocks = 8LL * kSmCount;
+    residue_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        s, x, (const long long *)keys, (unsigned long long *)out);
+    count_launch();
+    return cuda_status();
+}

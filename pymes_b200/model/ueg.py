@@ -563,11 +563,29 @@ def blocked_tiles(g_first, g_cnt, g_e0, g_en, tile_rows=64):
     return np.ascontiguousarray(tiles[np.argsort(-tiles[:, 3], kind="stable")])
 
 
+def linear_momenta(model):
+    """l(k) = n^2 x + n y + z (n = 2 imax + 1) of every orbital, the label the reference's index
+    lookup conserves (see :func:`momentum_groups`); cached on the model."""
+    lin = model.__dict__.get("_pmb_lin")
+    if lin is None:
+        k = model.k_int().astype(np.int64)
+        n = 2 * int(model.imax) + 1
+        lin = model.__dict__["_pmb_lin"] = n * n * k[:, 0] + n * k[:, 1] + k[:, 2]
+    return lin
+
+
+def momentum_rule(model, lo, ext, signs=SIGNS):
+    """``backend.Momentum`` of a tensor over the orbital ranges ``lo`` / ``ext`` with the given signs
+    (an integral block: (+,+,-,-); the Fock matrix: (+,-))."""
+    return bk.Momentum(linear_momenta(model), zip(lo, ext, signs))
+
+
 class MomentumGeom:
     """Where a STORED integral block sits in (p,q,r,s) orbital space: attached to the tensors
     ``UEG.eval_2b_blocks`` returns (``backend.tag_geom``) so that contractions whose structured
     operand is such a block can run on its diagonal momentum blocks (``pmb_blocked_contract``).
-    The structure is a property of the integral generator -- nothing is assumed about amplitudes."""
+    The structure is a property of the integral generator; the amplitudes' structure is derived
+    from it (``backend.Momentum``) or verified, never assumed."""
 
     def __init__(self, model, lo, ext):
         self.model, self.lo, self.ext = model, tuple(int(x) for x in lo), tuple(int(x) for x in ext)
@@ -584,6 +602,9 @@ class MomentumGeom:
             new_ext[dim] = int(n)
             sub = self._narrowed[key] = MomentumGeom(self.model, new_lo, new_ext)
         return sub
+
+    def momentum(self):
+        return momentum_rule(self.model, self.lo, self.ext)
 
     def partner_tables(self, S, y_axis):
         """For the stored block ``S`` (contiguous, this geometry) and one summed axis ``y_axis``:
@@ -687,6 +708,9 @@ class VirtualBlock(bk.GeneratedOperand):
             cache[key] = VirtualBlock(self.model, new_lo, new_ext, *self.tables, compressed=self.compressed,
                                       _packed=True)
         return cache[key]
+
+    def momentum(self):
+        return momentum_rule(self.model, self.lo, self.shape)
 
     def blocked_lists(self):
         """The block as the matrix [(p,q),(r,s)] is block diagonal in the (linearised) total

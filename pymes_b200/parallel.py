@@ -322,6 +322,9 @@ class ShardedCCSD(ccsd.CCSD):
         st["dtype_name"] = "float64"
         st["shift"] = level_shift
         e_mp2, T2 = mp2.solve_device(st["eps_i"], st["eps_a"], st["dV"]["ijab"], st["dV"]["abij"], level_shift)
+        # the exchanges (all-gather, row transpose) do not carry momentum rules yet: a sharded sweep
+        # starts from untagged amplitudes and keeps the dense ring products
+        bk.drop_momentum(T2)
         T1 = bk.zeros(nv, no)
         if amps is not None:
             T1, T2 = bk.asdev(amps[0]).contiguous(), bk.asdev(amps[1]).contiguous()

@@ -53,6 +53,22 @@ def _resolved(x):
     return x.wait_result() if hasattr(x, "wait_result") else x
 
 
+def block2(t, r0, nr, c0, nc):
+    """``t[r0:r0+nr, c0:c0+nc]`` as a view that keeps the momentum tag of ``t``."""
+    return bk.narrow(bk.narrow(t, 0, r0, nr), 1, c0, nc)
+
+
+def fock_rules(V_abij, no, nv):
+    """Momentum rules of the Fock matrix (+,-), T1 [a,i] and T2 [a,b,i,j] over the labels of the
+    tagged integral block ``V_abij``; None when the integrals carry no momentum tag."""
+    k = bk.momentum_of(V_abij)
+    if k is None:
+        return None
+    n = no + nv
+    return {"fock": k.with_axes([(0, n, 1), (0, n, -1)]), "t1": k.with_axes([(no, nv, 1), (0, no, -1)]),
+            "t2": k.with_axes([(no, nv, 1), (no, nv, 1), (0, no, -1), (0, no, -1)])}
+
+
 def doubles_residual(no, fock, T2, V_klij, V_ijab, V_abij, V_iajb, V_iabj, V_abcd,
                      is_dcd=False, is_bruekner=False, pp_ladder=None, shard=None):
     """R_abij for device tensors (reference ccd.py:164-254).
@@ -121,8 +137,8 @@ def doubles_residual(no, fock, T2, V_klij, V_ijab, V_abij, V_iajb, V_iabj, V_abc
             raise NotImplementedError("is_bruekner is not available in sharded runs")
         Xac, Xki = fock[no:, no:], fock[:no, :no]
     else:
-        Xac = bk.copy(sh.rows(fock[no:, no:], 0))
-        Xki = bk.copy(fock[:no, :no])
+        Xac = bk.copy(sh.rows(block2(fock, no, nv, no, nv), 0))
+        Xki = bk.copy(block2(fock, 0, no, 0, no))
     c = (1.0 if ccd else 0.5) if not is_bruekner else (0.5 if ccd else 0.0)
     if c != 0.0:
         ct("ac", [(-c, "adkl", Tta, "lkdc", V_ijab)], out=Xac, beta=1.0)

@@ -73,7 +73,7 @@ def t1_shared(T1, dV):
     out = {}
     for name, (spec, names) in SHARED_PRODUCTS.items():
         out[name] = bk.einsum(spec, *[src[n] for n in names.split()])
-    ones = torch.ones(T1.shape[1], dtype=bk.F64, device=T1.device)
+    ones = bk.ones(T1.shape[1])
     for name, (source, sub, view_sub) in SHARED_TRACES.items():
         out[name] = bk.einsum(view_sub + ",i->ab", bk.diag_view(out[source], sub, view_sub), ones)
     return out
@@ -124,10 +124,13 @@ def dressed_fock(no, fock, T1, dV, shared=None):
     """Device tensors in, dressed Fock (new tensor) out.  ccsd.py:226-288.  ``shared``: the
     result of :func:`t1_shared` for these amplitudes (computed here when not given)."""
     src = dict(dV)
-    src.update(t=T1, foo=fock[:no, :no], fvv=fock[no:, no:], fov=fock[:no, no:])
+    nv = fock.shape[0] - no
+    src.update(t=T1, foo=ccd.block2(fock, 0, no, 0, no), fvv=ccd.block2(fock, no, nv, no, nv),
+               fov=ccd.block2(fock, 0, no, no, nv))
     src.update(shared if shared is not None else t1_shared(T1, dV))
     out = bk.copy(fock)
-    views = {"ov": out[:no, no:], "vo": out[no:, :no], "oo": out[:no, :no], "vv": out[no:, no:]}
+    views = {"ov": ccd.block2(out, 0, no, no, nv), "vo": ccd.block2(out, no, nv, 0, no),
+             "oo": ccd.block2(out, 0, no, 0, no), "vv": ccd.block2(out, no, nv, no, nv)}
     for blk, rows in FOCK_TERMS.items():
         for coef, spec, names in rows:
             bk.einsum(spec, *[src[n] for n in names.split()], out=views[blk], alpha=coef, beta=1.0)
@@ -137,8 +140,7 @@ def dressed_fock(no, fock, T1, dV, shared=None):
 def dressed_block(key, T1, dV, skip_tau=False, shared=None):
     """One T1-dressed V block from the undressed dictionary.  ccsd.py:322-419.  ``shared``: the
     result of :func:`t1_shared` (needed by "iajb" / "iabj"; computed here when not given)."""
-    # a block without dressing terms (V_ijab) IS the stored block: its copy keeps the geometry tag
-    blk = bk.copy(dV[key]) if V_TERMS[key] else bk.copy_tagged(dV[key])
+    blk = bk.copy(dV[key])
     for coef, spec, source, is_tau in V_TERMS[key]:
         if skip_tau and is_tau:
             continue
@@ -156,8 +158,9 @@ def singles_residual(no, fock_dressed, T1, T2, dV):
     """R_ai from the dressed Fock matrix and the UNDRESSED integrals (ccsd.py:167-168, 423-438)."""
     Tt = bk.tilde(T2, swap_ij=True)
     src = dict(dV)
-    src.update(t=T1, Tt=Tt, fov=fock_dressed[:no, no:])
-    R1 = bk.copy(fock_dressed[no:, :no])
+    nv = fock_dressed.shape[0] - no
+    src.update(t=T1, Tt=Tt, fov=ccd.block2(fock_dressed, 0, no, no, nv))
+    R1 = bk.copy(ccd.block2(fock_dressed, no, nv, 0, no))
     for coef, spec, names in SINGLES_TERMS:
         bk.einsum(spec, *[src[n] for n in names.split()], out=R1, alpha=coef, beta=1.0)
     return R1
@@ -367,7 +370,15 @@ class CCSD(ccd.CCD):
         st["shift"] = level_shift
         e_mp2, T2 = mp2.solve_device(st["eps_i"], st["eps_a"], st["dV"]["ijab"], st["dV"]["abij"],
                                      level_shift)
-        T1 = bk.zeros(nv, no)
+        # Structure from outside is verified, never assumed.  The Fock matrix is checked on the host,
+        # where it already is.  The amplitudes start tagged only under a Hamiltonian that conserves
+        # momentum as a whole: with a one-body part that breaks the rule they break it from the first
+        # update on, and the sweeps then run dense from the start instead of switching after one.
+        rule = ccd.fock_rules(st["dV"]["abij"], no, nv)
+        if rule is not None and not bk.adopt_momentum(st["fock"], rule["fock"], host=fock_host):
+            rule = None
+        self._rules = rule
+        T1 = bk.zeros(nv, no, rule=rule["t1"] if rule is not None else None)
         st["amps_host"] = None
         if amps is not None:
             if isinstance(amps[0], torch.Tensor):
@@ -378,6 +389,11 @@ class CCSD(ccd.CCD):
                 st["amps_host"] = amps
                 T1, T2 = bk.asdev(amps[0]).contiguous(), bk.asdev(amps[1]).contiguous()
         st["T1"], st["T2"] = T1, T2
+        if rule is None:
+            bk.drop_momentum(T2)              # MP2 amplitudes of tagged integrals carry a derived rule
+        elif amps is not None:
+            bk.adopt_momentum(T1, rule["t1"])
+            bk.adopt_momentum(T2, rule["t2"])
         st["scal"] = bk.zeros(8)
         st["e_mp2"] = e_mp2
         st["iteration"] = 0
@@ -415,7 +431,7 @@ class CCSD(ccd.CCD):
             T1, T2 = self.mixer.mix([dT1, dT2], [T1, T2])
         st["T1"], st["T2"] = T1, T2
         bk.energy_doubles(T2, st["V_ijab_e"], scal, T1=T1)
-        bk.contract_terms("", [(2.0, "ia", fock[:no, no:], "ai", T1)], out=scal[4])
+        bk.contract_terms("", [(2.0, "ia", ccd.block2(fock, 0, no, no, T1.shape[0]), "ai", T1)], out=scal[4])
         s = scal.cpu().numpy()
         return float(s[4]), float(s[0]), float(s[1]), float(np.sqrt(s[2])), float(np.sqrt(s[3]))
 
@@ -429,6 +445,10 @@ class CCSD(ccd.CCD):
         t2 = t2_host if isinstance(t2_host, torch.Tensor) else torch.from_numpy(t2_host)
         st["T1"] = t1.to(bk.device(), non_blocking=True)
         st["T2"] = t2.to(bk.device(), non_blocking=True)
+        rule = getattr(self, "_rules", None)
+        if rule is not None:
+            bk.adopt_momentum(st["T1"], rule["t1"])
+            bk.adopt_momentum(st["T2"], rule["t2"])
         out = self.sweep()
         t1.copy_(st["T1"], non_blocking=True)
         t2.copy_(st["T2"], non_blocking=True)
