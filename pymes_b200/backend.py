@@ -684,6 +684,10 @@ def adopt_momentum(t, key, host=None):
         ok = not np.any(host[total != 0] != 0)           # NaN != 0: not adopted
         _set_momentum(t, key if ok else None)
         return ok
+    if t.numel() == 0:
+        # no element can break the rule (and pmb_momentum_residue takes no extent of 0)
+        _set_momentum(t, key)
+        return True
     labels = torch.from_numpy(np.concatenate([key.labels(d) for d in range(t.dim())])).to(device())
     res = zeros(1)
     _lib.check(_lib.load().pmb_momentum_residue(t.dim(), _lib.I64x4(*_pad4r(t.shape, 1)),
