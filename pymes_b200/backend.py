@@ -1313,12 +1313,22 @@ def update_singles(eps_i, eps_a, shift, delta, R1, T1):
     return dT1
 
 
+def _flat(what, t, shape):
+    """Raise unless ``t`` is a contiguous tensor of ``shape``: the kernels index it flat."""
+    if tuple(t.shape) != tuple(shape) or not t.is_contiguous():
+        raise ValueError("%s must be a contiguous tensor of shape %s (got shape %s, strides %s)"
+                         % (what, tuple(shape), tuple(t.shape), tuple(t.stride())))
+
+
 def energy_doubles(T2, V_ijab, scal, T1=None, mp2_form=False, rows=None):
     """scal[0:3] = (E_direct, E_exchange, |T2|^2) on the device (partial sums over the local
     row block when ``rows=(a_lo, na)``; V_ijab and T1 are always the full tensors)."""
     lib = _lib.load()
     nv, no = T2.shape[1], T2.shape[2]
     a_lo, na = rows if rows is not None else (0, nv)
+    _flat("energy_doubles: T2", T2, (na, nv, no, no))
+    if T1 is not None:
+        _flat("energy_doubles: T1", T1, (nv, no))
     ws = scratch().reduce_ws()
     _lib.check(lib.pmb_energy_doubles(no, nv, a_lo, na, _ptr(T2), _ptr(T1) if T1 is not None else None,
                                       _ptr(V_ijab), _lib.I64x4(*V_ijab.stride()), int(mp2_form), _ptr(scal),
@@ -1329,6 +1339,7 @@ def energy_doubles(T2, V_ijab, scal, T1=None, mp2_form=False, rows=None):
 def tilde(T2, swap_ij=False):
     lib = _lib.load()
     nv, no = T2.shape[0], T2.shape[2]
+    _flat("tilde: T2", T2, (nv, nv, no, no))
     Tt = torch.empty_like(T2)
     k = momentum_of(T2)
     _lib.check(lib.pmb_tilde(no, nv, _ptr(T2), _ptr(Tt), int(swap_ij), _stream()), "pmb_tilde")
@@ -1341,8 +1352,10 @@ def sym_baji(Ex, R=None, accumulate=True):
     """R (+)= Ex + Ex^{baji}."""
     lib = _lib.load()
     nv, no = Ex.shape[0], Ex.shape[2]
+    _flat("sym_baji: Ex", Ex, (nv, nv, no, no))
     if R is None:
         R, accumulate = torch.empty_like(Ex), False
+    _flat("sym_baji: R", R, (nv, nv, no, no))
     k, chain = momentum_of(Ex), _chain(R)
     if k is not None and (k.permute((1, 0, 3, 2)) != k or (accumulate and momentum_of(R) != k)):
         k = None

@@ -123,7 +123,7 @@ class FakeLib:
         B, _, _ = _gather(d.B, (bk_[:, None] + bx[None, :]).reshape(-1))
         val = d.alpha * (vec @ B.reshape(len(vk), len(bx)))
         old, win, lo = _gather(d.out, ox)
-        win[ox - lo] = val + (d.beta * old if d.beta != 0.0 else 0.0)
+        win[ox - lo] = val if d.beta == 0.0 else val + d.beta * old
         return 0
 
     def pmb_bdot(self, dref, stream):
@@ -140,7 +140,7 @@ class FakeLib:
         B, _, _ = _gather(d.B, (bi[:, None] + br[None, :]).reshape(-1))
         val = d.alpha * (A * B).reshape(len(oi), -1).sum(axis=1)
         old, win, lo = _gather(d.out, oi)
-        win[oi - lo] = val + (d.beta * old if d.beta != 0.0 else 0.0)
+        win[oi - lo] = val if d.beta == 0.0 else val + d.beta * old
         return 0
 
     # ---- elementwise ------------------------------------------------
@@ -151,7 +151,8 @@ class FakeLib:
         oo = _offsets(e[::-1], [out_str[i] for i in range(4)][::-1])
         src, _, _ = _gather(_val(inp), oi)
         old, win, lo = _gather(_val(out), oo)
-        win[oo - lo] = alpha * src + (beta * old if beta != 0.0 else 0.0)
+        # beta = 0: alpha x is stored as it is (a -0.0 stays -0.0) and the output is never read
+        win[oo - lo] = alpha * src if beta == 0.0 else alpha * src + beta * old
         return 0
 
     @staticmethod
@@ -174,7 +175,9 @@ class FakeLib:
         n = na * nv * no * no
         D, e_i, e_a = self._denoms(no, nv, ei, ea, shift)
         if denom_mode:
-            D = np.einsum("i,j,a,b->abij", e_i, e_i, -e_a, -e_a) + shift
+            # the product in the kernel's order: ((e_i e_j) (-e_a)) (-e_b)
+            D = (((e_i[None, None, :, None] * e_i[None, None, None, :]) * -e_a[:, None, None, None])
+                 * -e_a[None, :, None, None]) + shift
         d = _window(_val(R), n) * (1.0 / D[a_lo:a_lo + na]).reshape(-1)
         _window(_val(dT), n)[:] = d
         _window(_val(T2), n)[:] += delta * d
@@ -211,6 +214,8 @@ class FakeLib:
         return 0
 
     def pmb_tilde(self, no, nv, T2, Tt, swap_ij, stream):
+        if no <= 0 or nv <= 0 or _val(T2) == _val(Tt):
+            return -1                     # PMB_E_BADARG, as the library does
         self.launches += 1
         n = nv * nv * no * no
         t = _window(_val(T2), n).reshape(nv, nv, no, no)
@@ -219,6 +224,8 @@ class FakeLib:
         return 0
 
     def pmb_sym_baji(self, no, nv, Ex, R, accumulate, stream):
+        if no <= 0 or nv <= 0 or _val(Ex) == _val(R):
+            return -1
         self.launches += 1
         n = nv * nv * no * no
         e = _window(_val(Ex), n).reshape(nv, nv, no, no)
@@ -228,7 +235,7 @@ class FakeLib:
         return 0
 
     def pmb_dots(self, nvec, X, Y, n, out, ws, wsb, stream):
-        if not 1 <= nvec <= 16:
+        if not 1 <= nvec <= 16 or n <= 0:
             return -1                     # PMB_E_BADARG, as the library does
         self.launches += 2
         y = _window(_val(Y), n)
@@ -238,7 +245,7 @@ class FakeLib:
         return 0
 
     def pmb_lincomb(self, nvec, c, X, n, beta, out, stream):
-        if not 1 <= nvec <= 16:
+        if not 1 <= nvec <= 16 or n <= 0:
             return -1
         self.launches += 1
         o = _window(_val(out), n)

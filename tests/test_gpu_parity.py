@@ -998,7 +998,9 @@ def test_elementwise_kernels_pair_rows_and_streams(no, nv):
     """Round-2 forms of the HBM-bound kernels: T-tilde and Ex + Ex^{baji} by row PAIRS (a,b),(b,a),
     the energy streaming an [a,b,i,j]-stored V_ijab (whole tensor and a row block), the strided copy
     with its 32-bit inner index split -- all against numpy, bit for bit where no sum is involved.
-    o = 50 exceeds the shared-memory row buffers of sym_baji: the element-per-thread kernels run."""
+    Every o here runs the row-pair kernels: o = 50 still fits the two shared-memory rows of
+    sym_baji (40000 of 49152 bytes).  The element-per-thread fallbacks (o >= 56 for sym_baji,
+    o >= 65 for T-tilde) are covered in test_elementwise_edges.py."""
     from pymes_b200 import backend as bk
     from pymes_b200.solver import ccsd
     rng = np.random.default_rng(no * 100 + nv)
