@@ -998,29 +998,32 @@ def _try_gather(out_sub, terms, out, beta):
 
 def _group_term(out_sub, term):
     """``(alpha, sa, A, sb, B, sigma)`` if this term can go to ``pmb_group_contract``: both operands
-    stored tensors with a live momentum rule, and the split 2 | 2 | 2 (two output indices from A,
-    two summed, two output indices from B) with the summed axes cancelling under one sign sigma.
-    Else None."""
+    stored tensors of rank 1-4 with a live momentum rule that the term conserves (``_term_keys``).
+    Every index of A is an output index (a row) or summed with B (an entry), every other index of B
+    is an output index (a column), and there is at least one output index.  A summed axis with a
+    non-zero sign on both operands fixes the sign sigma; a term whose summed axes all have sign 0
+    (a trace with :func:`ones`) is left to the other paths.  Without summed axes (an outer
+    product) only group 0 exists and sigma = 1.  Else None."""
     if not _BLOCKED[0]:
         return None
     alpha, sa, A, sb, B = term
-    if not (isinstance(A, torch.Tensor) and isinstance(B, torch.Tensor)):
+    if not (isinstance(A, torch.Tensor) and isinstance(B, torch.Tensor)) or not out_sub:
         return None
-    if len(sa) != 4 or len(sb) != 4 or len(out_sub) != 4 or A.dim() != 4 or B.dim() != 4:
+    if not (1 <= len(sa) <= 4 and 1 <= len(sb) <= 4) or A.dim() != len(sa) or B.dim() != len(sb):
         return None
-    if len(set(sa)) != 4 or len(set(sb)) != 4 or len(set(out_sub)) != 4:
+    if len(set(sa)) != len(sa) or len(set(sb)) != len(sb) or len(set(out_sub)) != len(out_sub):
         return None
     ka, kb = momentum_of(A), momentum_of(B)
-    if ka is None or kb is None or not _term_keys(out_sub, sa, ka, sb, kb):
+    if ka is None or kb is None or len(ka.axes) != len(sa) or len(kb.axes) != len(sb):
         return None
-    rows = [ch for ch in sa if ch in out_sub]
-    cols = [ch for ch in sb if ch in out_sub]
-    ents = [ch for ch in sa if ch not in out_sub]
-    if len(rows) != 2 or len(cols) != 2 or sorted(ents) != sorted(ch for ch in sb if ch not in out_sub):
+    if not _term_keys(out_sub, sa, ka, sb, kb):
         return None
-    ga, gb = ka.axes[sa.index(ents[0])][2], kb.axes[sb.index(ents[0])][2]
-    if ga == 0 or gb == 0:
+    ents = [ch for ch in sa if ch in sb]
+    signs = [(ka.axes[sa.index(ch)][2], kb.axes[sb.index(ch)][2]) for ch in ents]
+    signs = [(ga, gb) for ga, gb in signs if ga != 0 and gb != 0]
+    if ents and not signs:
         return None
+    ga, gb = signs[0] if signs else (1, -1)
     return float(alpha), sa, A, sb, B, (-1 if ga == gb else 1)
 
 
@@ -1028,60 +1031,86 @@ _GROUP_CACHE = {}
 GROUP_TILE = 32          # rows / columns per tile of pmb_group_contract (its GT)
 
 
-def _sorted_side(labels):
-    """Stable order of a side's flat positions by label, its distinct labels, first positions, counts."""
-    order = np.argsort(labels, kind="stable")
-    keys, first, cnt = np.unique(labels[order], return_index=True, return_counts=True)
-    return order, keys, first, cnt
+def _side_keys(k, axes, sign):
+    """The distinct labels of one side (``sign`` times the sum of its axes' labels), grown one axis
+    at a time so that the labels of a long side (o.v^2 members) are never all formed."""
+    keys = np.zeros(1, dtype=np.int64)
+    for d in axes:
+        keys = np.unique(np.add.outer(keys, np.unique(k.labels(d))))
+    return sign * keys
+
+
+def _side_members(k, axes, sign, common):
+    """Flat positions (C order over ``axes``) of the side's members whose label is in ``common``,
+    stably sorted by label, with each group's first index and count in that list."""
+    lab = np.zeros(1, dtype=np.int64)
+    for d in axes:
+        lab = np.add.outer(lab, sign * k.labels(d)).reshape(-1)
+    pos = np.flatnonzero(np.isin(lab, common))
+    pos = pos[np.argsort(lab[pos], kind="stable")]
+    _keys, first, cnt = np.unique(lab[pos], return_index=True, return_counts=True)
+    return pos, first, cnt
+
+
+def _side_offsets(pos, ext, *strides):
+    """Element offsets of flat positions ``pos`` over extents ``ext``, one array per stride set."""
+    idx = np.unravel_index(pos, ext) if ext else ()
+    offs = []
+    for st in strides:
+        o = np.zeros(len(pos), dtype=np.int64)
+        for i, s_ in zip(idx, st):
+            o += i.astype(np.int64) * int(s_)
+        offs.append(o)
+    return offs
 
 
 def _group_plan(out_sub, g, out):
     """Device lists and tiles of one group term, cached by value: the three sides' momentum labels
-    and the strides of A, B and C (intermediates are new tensors every sweep and hit the cache)."""
+    and the strides of A, B and C (intermediates are new tensors every sweep and hit the cache).
+    A side without axes (rows of a matrix-vector product, entries of an outer product) has one
+    member, label 0 and offset 0.  Only members of groups common to all three sides are listed;
+    when there is none, the plan has no tile and nothing is uploaded."""
     _alpha, sa, A, sb, B, sigma = g
     ka, kb = momentum_of(A), momentum_of(B)
-    rows = [sa.index(ch) for ch in sa if ch in out_sub]
-    ents = [sa.index(ch) for ch in sa if ch not in out_sub]
-    cols = [sb.index(ch) for ch in sb if ch in out_sub]
+    rows = [d for d, ch in enumerate(sa) if ch in out_sub]
+    ents = [d for d, ch in enumerate(sa) if ch not in out_sub]
+    cols = [d for d, ch in enumerate(sb) if ch in out_sub]
     b_ents = [sb.index(sa[d]) for d in ents]
     cstr = dict(zip(out_sub, out.stride()))
-    key = (ka.lin_key, tuple(ka.axes[d] for d in rows + ents), tuple(kb.axes[d] for d in cols), sigma,
+    key = (ka.lin_key, kb.lin_key, tuple(ka.axes[d] for d in rows + ents), tuple(kb.axes[d] for d in cols), sigma,
            tuple(A.stride(d) for d in rows + ents), tuple(B.stride(d) for d in b_ents + cols),
            tuple(cstr[sa[d]] for d in rows), tuple(cstr[sb[d]] for d in cols), str(out.device))
     plan = _GROUP_CACHE.get(key)
     if plan is not None:
         return plan
-    outer = lambda x, y: (x[:, None] + y[None, :]).reshape(-1)
-    r_lab = outer(ka.labels(rows[0]), ka.labels(rows[1]))
-    e_lab = -outer(ka.labels(ents[0]), ka.labels(ents[1]))
-    c_lab = -sigma * outer(kb.labels(cols[0]), kb.labels(cols[1]))
-    r_ord, r_key, r_first, r_cnt = _sorted_side(r_lab)
-    e_ord, e_key, e_first, e_cnt = _sorted_side(e_lab)
-    c_ord, c_key, c_first, c_cnt = _sorted_side(c_lab)
-    common = np.intersect1d(np.intersect1d(r_key, e_key, assume_unique=True), c_key, assume_unique=True)
-    ri, ei, ci = (np.searchsorted(k, common) for k in (r_key, e_key, c_key))
+    sides = ((ka, rows, 1), (ka, ents, -1), (kb, cols, -sigma))
+    common = np.intersect1d(_side_keys(*sides[0]), _side_keys(*sides[2]))
+    if len(common):
+        common = np.intersect1d(common, _side_keys(*sides[1]))
+    if not len(common):
+        plan = dict(tiles=torch.zeros((0, 6), dtype=torch.int32), n_tiles=0, flops=0.0)
+        _GROUP_CACHE[key] = plan
+        return plan
+    (r_pos, r_first, r_cnt), (e_pos, e_first, e_cnt), (c_pos, c_first, c_cnt) = (
+        _side_members(*s_, common) for s_ in sides)
     tiles = []
-    for g0, (r0, rn, e0, en, c0, cn) in enumerate(zip(r_first[ri], r_cnt[ri], e_first[ei], e_cnt[ei],
-                                                     c_first[ci], c_cnt[ci])):
+    for r0, rn, e0, en, c0, cn in zip(r_first, r_cnt, e_first, e_cnt, c_first, c_cnt):
         for rt in range(0, int(rn), GROUP_TILE):
             for ct_ in range(0, int(cn), GROUP_TILE):
                 tiles.append((r0 + rt, min(GROUP_TILE, rn - rt), e0, en, c0 + ct_, min(GROUP_TILE, cn - ct_)))
     tiles = np.asarray(tiles, dtype=np.int32).reshape(-1, 6)
-    n1 = lambda d, t: int(t.shape[d])
     dev = out.device
     up = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64)).to(dev)
-    ra, rb_ = r_ord // n1(rows[1], A), r_ord % n1(rows[1], A)
-    ea, eb = e_ord // n1(ents[1], A), e_ord % n1(ents[1], A)
-    ca, cb = c_ord // n1(cols[1], B), c_ord % n1(cols[1], B)
+    a_row, c_row = _side_offsets(r_pos, [A.shape[d] for d in rows], [A.stride(d) for d in rows],
+                                 [cstr[sa[d]] for d in rows])
+    a_ent, b_ent = _side_offsets(e_pos, [A.shape[d] for d in ents], [A.stride(d) for d in ents],
+                                 [B.stride(d) for d in b_ents])
+    b_col, c_col = _side_offsets(c_pos, [B.shape[d] for d in cols], [B.stride(d) for d in cols],
+                                 [cstr[sb[d]] for d in cols])
     plan = dict(
-        a_row=up(ra * A.stride(rows[0]) + rb_ * A.stride(rows[1])),
-        a_ent=up(ea * A.stride(ents[0]) + eb * A.stride(ents[1])),
-        b_ent=up(ea * B.stride(b_ents[0]) + eb * B.stride(b_ents[1])),
-        b_col=up(ca * B.stride(cols[0]) + cb * B.stride(cols[1])),
-        c_row=up(ra * cstr[sa[rows[0]]] + rb_ * cstr[sa[rows[1]]]),
-        c_col=up(ca * cstr[sb[cols[0]]] + cb * cstr[sb[cols[1]]]),
+        a_row=up(a_row), a_ent=up(a_ent), b_ent=up(b_ent), b_col=up(b_col), c_row=up(c_row), c_col=up(c_col),
         tiles=torch.from_numpy(np.ascontiguousarray(tiles)).to(dev), n_tiles=len(tiles),
-        flops=2.0 * float((r_cnt[ri] * e_cnt[ei] * c_cnt[ci]).sum()))
+        flops=2.0 * float((r_cnt * e_cnt * c_cnt).sum()))
     _GROUP_CACHE[key] = plan
     return plan
 
@@ -1096,6 +1125,11 @@ def _run_group(out_sub, g, out, beta):
     elif beta != 1.0:
         axpby(beta, out, 0.0, out)
     d = _lib.Group()
+    if not plan["n_tiles"]:
+        # no group is common to the three sides: the product is zero and nothing is launched
+        # (pmb_group_contract returns before it reads a table)
+        _lib.check(_lib.load().pmb_group_contract(C.byref(d), _stream()), "pmb_group_contract")
+        return
     d.A, d.B, d.C = A.data_ptr(), B.data_ptr(), out.data_ptr()
     d.a_row, d.a_ent, d.b_ent = plan["a_row"].data_ptr(), plan["a_ent"].data_ptr(), plan["b_ent"].data_ptr()
     d.b_col, d.c_row, d.c_col = plan["b_col"].data_ptr(), plan["c_row"].data_ptr(), plan["c_col"].data_ptr()
@@ -1113,7 +1147,7 @@ def _run_group(out_sub, g, out, beta):
 
 def _try_blocked(out_sub, terms, out, beta):
     """Terms with momentum structure are evaluated on their diagonal blocks only: both operands
-    with a live momentum rule and a 2 | 2 | 2 split by ``pmb_group_contract`` (``_group_term``), a
+    with a live momentum rule by ``pmb_group_contract`` (``_group_term``), a
     stored or generated integral block times a dense operand by ``pmb_blocked_contract``
     (``_blocked_term``).  The other terms of the same call (e.g. the hole-hole ladder next to the
     particle-particle one, ccd.py:185-187) keep the dense kernel.  Returns the result, or None when
@@ -1188,6 +1222,10 @@ def _contract_terms(out_sub, terms, out, beta):
     if out is not None and out.device != device():
         raise RuntimeError("pymes_b200: output tensor lives on %s, the kernels write to %s "
                            "(there is no CPU fallback)" % (out.device, device()))
+    # a term whose operands both carry a live rule runs on its momentum groups, however cheap the
+    # matrix-vector or gather kernel would be: the group plan skips every product the rules make zero
+    if any(_group_term(out_sub, t) is not None for t in terms):
+        return _try_blocked(out_sub, terms, out, beta)
     res = _try_gemv(out_sub, terms, out, beta)
     if res is not None:
         return res

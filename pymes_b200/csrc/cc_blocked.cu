@@ -289,11 +289,19 @@ extern "C" int pmb_gather_expand(const pmb_gather_t *d, pmb_stream_t stream) {
 // shared memory and accumulates with FP64 FMA (2 x 2 outputs per thread).  The work per product is
 // a few 10^7 flop, so the tensor cores would buy nothing here; what matters is that no zero is
 // read.  Each C element belongs to one tile: deterministic, no atomics.
+//
+// A tile of at most GE outputs with more than GK entries (a diagonal build such as "kcdl,cdil->ki":
+// 1 x 1 tiles of ~8.8e3 entries at 54 electrons) would walk its slabs on a single thread.  Such a
+// tile takes the entry-split form instead: each of the GNT threads sums every GNT-th entry, then a
+// fixed-order tree in shared memory combines the partial sums -- still deterministic, no atomics.
+// The form is chosen per tile from (rn, en, cn), so the host plan and the C ABI do not know it.
 // ---------------------------------------------------------------------------
 namespace pmb {
 namespace {
 
-constexpr int GT = 32, GK = 32, GNT = 256;
+constexpr int GT = 32, GK = 32, GNT = 256, GE = 4;
+static_assert(GE * GNT <= GK * (GT + 1), "the entry-split partial sums reuse As");
+static_assert((GNT & (GNT - 1)) == 0, "tree reduction over GNT threads");
 
 __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_group_t p) {
     __shared__ double As[GK][GT + 1];
@@ -311,6 +319,32 @@ __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_
         const bool ok = j < cn;
         s_bc[j] = ok ? p.b_col[c0 + j] : 0;
         s_cc[j] = ok ? p.c_col[c0 + j] : 0;
+    }
+    const int no = rn * cn;
+    if (en > GK && no <= GE) {
+        __syncthreads();                          // offsets staged
+        double acc[GE];
+#pragma unroll
+        for (int o = 0; o < GE; ++o) acc[o] = 0.0;
+        for (int k = tid; k < en; k += GNT) {
+            const long long ae = __ldg(p.a_ent + e0 + k), be = __ldg(p.b_ent + e0 + k);
+#pragma unroll
+            for (int o = 0; o < GE; ++o)
+                if (o < no) acc[o] = fma(__ldg(p.A + s_ar[o / cn] + ae), __ldg(p.B + be + s_bc[o % cn]), acc[o]);
+        }
+        double *red = &As[0][0];                  // [GE][GNT]
+#pragma unroll
+        for (int o = 0; o < GE; ++o) red[o * GNT + tid] = acc[o];
+        for (int w = GNT / 2; w > 0; w >>= 1) {
+            __syncthreads();
+            if (tid < w) {
+#pragma unroll
+                for (int o = 0; o < GE; ++o) red[o * GNT + tid] += red[o * GNT + tid + w];
+            }
+        }
+        __syncthreads();
+        if (tid < no) p.C[s_cr[tid / cn] + s_cc[tid % cn]] += p.alpha * red[tid * GNT];
+        return;
     }
     const int tx = tid % 16, ty = tid / 16;       // columns tx, tx+16; rows ty, ty+16
     double acc[2][2] = {{0.0, 0.0}, {0.0, 0.0}};
