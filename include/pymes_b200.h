@@ -433,6 +433,22 @@ typedef struct {
 } pmb_group_t;
 int pmb_group_contract(const pmb_group_t *d, pmb_stream_t stream);
 
+/* The same product for n_batch right-hand sides at once (Davidson / FEAST     */
+/* blocks): right-hand side b reads A + b*a_bstr, B + b*b_bstr and writes        */
+/* C + b*c_bstr with the one set of lists and tiles in g.  A batch stride of 0  */
+/* shares that operand between all right-hand sides (c_bstr only when          */
+/* n_batch == 1).  One CTA per (tile, right-hand side); same summation order    */
+/* as pmb_group_contract, no atomics.  1 <= n_batch <= 65535.                   */
+typedef struct {
+    pmb_group_t g;
+    int32_t n_batch;
+    int32_t _pad;
+    int64_t a_bstr;
+    int64_t b_bstr;
+    int64_t c_bstr;
+} pmb_group_batched_t;
+int pmb_group_contract_batched(const pmb_group_batched_t *d, pmb_stream_t stream);
+
 /* Momentum residue of a strided tensor of rank 1..4:                          */
 /*   out[0] = max |x[i0,..]| over the elements with sum_d key_d[i_d] != 0,       */
 /* key_d = keys + (ext[0] + .. + ext[d-1]) (per-axis signed momentum labels,    */

@@ -77,6 +77,11 @@ class Group(C.Structure):
                 ("alpha", C.c_double)]
 
 
+class GroupBatched(C.Structure):
+    _fields_ = [("g", Group), ("n_batch", C.c_int32), ("_pad", C.c_int32), ("a_bstr", C.c_int64),
+                ("b_bstr", C.c_int64), ("c_bstr", C.c_int64)]
+
+
 _SIGS = {
     "pmb_version": (C.c_int, []),
     "pmb_device_info": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]),
@@ -117,6 +122,7 @@ _SIGS = {
     "pmb_blocked_contract": (C.c_int, [C.POINTER(Blocked), C.c_void_p]),
     "pmb_gather_expand": (C.c_int, [C.POINTER(Gather), C.c_void_p]),
     "pmb_group_contract": (C.c_int, [C.POINTER(Group), C.c_void_p]),
+    "pmb_group_contract_batched": (C.c_int, [C.POINTER(GroupBatched), C.c_void_p]),
     "pmb_momentum_residue": (C.c_int, [C.c_int, I64x4, I64x4, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pmb_synth_block": (C.c_int, [C.c_int, C.c_ulonglong, C.c_double, C.c_void_p, I32x4, I32x4, C.c_void_p,
                                   C.c_void_p]),

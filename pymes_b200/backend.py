@@ -591,32 +591,41 @@ def _column_groups(n_sub, ext, bstr, cstr):
 # --------------------------------------------------------------------------
 class Momentum:
     """Selection rule of a tensor: ``x[i_0, i_1, ..]`` can be non-zero only where
-    ``sum_d sign_d * lin[lo_d + i_d] == 0``, ``lin`` the linearised momentum of every orbital
+    ``sum_d sign_d * lin[lo_d + i_d] == total``, ``lin`` the linearised momentum of every orbital
     (``model.ueg.momentum_groups``) and one ``(lo, ext, sign)`` per axis.  A stored UEG integral block
-    has signs (+,+,-,-); contractions, linear combinations and index swaps of tensors with such rules
-    have one as well (:func:`contract_terms` derives it), and a tensor from outside gets one only by
-    :func:`adopt_momentum`, which checks it.  A sign 0 leaves its axis unconstrained.  Kept in a
-    normal form (first non-zero sign positive): rules equal up to an overall sign compare equal."""
+    has signs (+,+,-,-) and total 0; an excitation vector of one total-momentum sector
+    (``model.ueg.excitation_sector``) has total l(K).  Contractions, linear combinations and index
+    swaps of tensors with such rules have one as well (:func:`contract_terms` derives it), and a
+    tensor from outside gets one only by :func:`adopt_momentum`, which checks it.  A sign 0 leaves
+    its axis unconstrained.  Kept in a normal form (first non-zero sign positive, the total flipped
+    with the signs): rules equal up to an overall sign compare equal."""
 
-    __slots__ = ("lin", "lin_key", "axes")
+    __slots__ = ("lin", "lin_key", "axes", "total")
 
-    def __init__(self, lin, axes, lin_key=None):
+    def __init__(self, lin, axes, lin_key=None, total=0):
         axes = tuple((int(lo), int(n), int(sg)) for lo, n, sg in axes)
+        total = int(total)
         first = next((sg for _lo, _n, sg in axes if sg), 1)
         if first < 0:
             axes = tuple((lo, n, -sg) for lo, n, sg in axes)
+            total = -total
         self.lin = lin
         self.lin_key = lin_key if lin_key is not None else (lin.tobytes() if lin is not None else None)
         self.axes = axes
+        self.total = total
 
     def __eq__(self, other):
-        return isinstance(other, Momentum) and self.axes == other.axes and self.lin_key == other.lin_key
+        return isinstance(other, Momentum) and self.axes == other.axes and self.total == other.total \
+            and self.lin_key == other.lin_key
 
     def __hash__(self):
-        return hash((self.axes, self.lin_key))
+        return hash((self.axes, self.total, self.lin_key))
 
     def with_axes(self, axes):
-        return Momentum(self.lin, axes, self.lin_key)
+        return Momentum(self.lin, axes, self.lin_key, self.total)
+
+    def with_total(self, total):
+        return Momentum(self.lin, self.axes, self.lin_key, total)
 
     def narrow(self, dim, lo, n):
         axes = list(self.axes)
@@ -627,12 +636,18 @@ class Momentum:
     def permute(self, dims):
         return self.with_axes([self.axes[d] for d in dims])
 
-    def labels(self, d):
-        """Signed momentum labels ``sign * lin[lo:lo+ext]`` of axis ``d`` (int64)."""
+    def signed(self, d):
+        """Signed momentum labels ``sign * lin[lo:lo+ext]`` of axis ``d`` (int64), without the total."""
         lo, n, sg = self.axes[d]
         if sg == 0:
             return np.zeros(n, dtype=np.int64)
         return sg * np.asarray(self.lin[lo:lo + n], dtype=np.int64)
+
+    def labels(self, d):
+        """Labels of axis ``d`` such that an allowed element's labels sum to 0: the signed labels,
+        with the total subtracted from those of axis 0 (what ``pmb_momentum_residue`` checks)."""
+        lab = self.signed(d)
+        return lab - self.total if d == 0 and self.total else lab
 
 
 def _set_momentum(t, key):
@@ -741,7 +756,8 @@ def _term_keys(out_sub, sa, ka, sb, kb):
     """The rules the product ``einsum(sa, sb -> out_sub)`` of operands with rules ``ka`` / ``kb``
     satisfies: with one sign sigma for the whole term, every summed axis must cancel
     (``sign_a + sigma * sign_b == 0`` over the same orbitals); the output axes then carry the signs
-    of A and sigma times those of B.  Both sigmas when nothing constrains it (outer products)."""
+    of A and sigma times those of B, and the total ``total_A + sigma * total_B``.  Both sigmas when
+    nothing constrains it (outer products)."""
     if ka.lin_key is not None and kb.lin_key is not None and ka.lin_key != kb.lin_key:
         return set()
     lin, lin_key = (ka.lin, ka.lin_key) if ka.lin_key is not None else (kb.lin, kb.lin_key)
@@ -763,7 +779,7 @@ def _term_keys(out_sub, sa, ka, sb, kb):
     if any(ch not in sa and ch not in out_sub for ch in sb) or any(ch not in xa and ch not in xb for ch in out_sub):
         return set()
     return {Momentum(lin, [xa[ch] if ch in xa else (xb[ch][0], xb[ch][1], sg * xb[ch][2]) for ch in out_sub],
-                     lin_key) for sg in sigmas}
+                     lin_key, ka.total + sg * kb.total) for sg in sigmas}
 
 
 def _derive(out_sub, terms, old, accumulate):
@@ -1031,21 +1047,22 @@ _GROUP_CACHE = {}
 GROUP_TILE = 32          # rows / columns per tile of pmb_group_contract (its GT)
 
 
-def _side_keys(k, axes, sign):
-    """The distinct labels of one side (``sign`` times the sum of its axes' labels), grown one axis
-    at a time so that the labels of a long side (o.v^2 members) are never all formed."""
+def _side_keys(k, axes, sign, shift=0):
+    """The distinct labels of one side (``sign`` times the sum of its axes' signed labels, plus
+    ``shift``), grown one axis at a time so that the labels of a long side (o.v^2 members) are
+    never all formed."""
     keys = np.zeros(1, dtype=np.int64)
     for d in axes:
-        keys = np.unique(np.add.outer(keys, np.unique(k.labels(d))))
-    return sign * keys
+        keys = np.unique(np.add.outer(keys, np.unique(k.signed(d))))
+    return sign * keys + shift
 
 
-def _side_members(k, axes, sign, common):
+def _side_members(k, axes, sign, shift, common):
     """Flat positions (C order over ``axes``) of the side's members whose label is in ``common``,
     stably sorted by label, with each group's first index and count in that list."""
-    lab = np.zeros(1, dtype=np.int64)
+    lab = np.full(1, shift, dtype=np.int64)
     for d in axes:
-        lab = np.add.outer(lab, sign * k.labels(d)).reshape(-1)
+        lab = np.add.outer(lab, sign * k.signed(d)).reshape(-1)
     pos = np.flatnonzero(np.isin(lab, common))
     pos = pos[np.argsort(lab[pos], kind="stable")]
     _keys, first, cnt = np.unique(lab[pos], return_index=True, return_counts=True)
@@ -1078,12 +1095,15 @@ def _group_plan(out_sub, g, out):
     b_ents = [sb.index(sa[d]) for d in ents]
     cstr = dict(zip(out_sub, out.stride()))
     key = (ka.lin_key, kb.lin_key, tuple(ka.axes[d] for d in rows + ents), tuple(kb.axes[d] for d in cols), sigma,
+           ka.total, kb.total,
            tuple(A.stride(d) for d in rows + ents), tuple(B.stride(d) for d in b_ents + cols),
            tuple(cstr[sa[d]] for d in rows), tuple(cstr[sb[d]] for d in cols), str(out.device))
     plan = _GROUP_CACHE.get(key)
     if plan is not None:
         return plan
-    sides = ((ka, rows, 1), (ka, ents, -1), (kb, cols, -sigma))
+    # group label g = R - t_A = -E_A = sigma (t_B - C_B): R, E_A the signed row / entry sums of A,
+    # C_B the column sum of B, t_A / t_B the totals (A: R + E_A = t_A; B: -sigma E_A + C_B = t_B)
+    sides = ((ka, rows, 1, -ka.total), (ka, ents, -1, 0), (kb, cols, -sigma, sigma * kb.total))
     common = np.intersect1d(_side_keys(*sides[0]), _side_keys(*sides[2]))
     if len(common):
         common = np.intersect1d(common, _side_keys(*sides[1]))
@@ -1145,15 +1165,91 @@ def _run_group(out_sub, g, out, beta):
     _lib.check(rc, "pmb_group_contract")
 
 
+def _batched_group_term(out_sub, term):
+    """``(alpha, sa, A, sb, B, g, n_batch, a_bstr, b_bstr)`` if this term is a group product
+    (:func:`_group_term`) repeated over a batch axis: the output's leading index ``r`` is held by A
+    and / or B on an axis of sign 0 (stacked right-hand sides, :func:`stack`), and the product of
+    one slice qualifies.  ``g`` is that slice's group term (views of right-hand side 0, tagged with
+    the rules less the batch axis); a stride of 0 marks the operand without ``r``.  Else None."""
+    if not _BLOCKED[0]:
+        return None
+    alpha, sa, A, sb, B = term
+    if not (isinstance(A, torch.Tensor) and isinstance(B, torch.Tensor)) or len(out_sub) < 2:
+        return None
+    r = out_sub[0]
+    if r not in sa and r not in sb:
+        return None
+    sliced, n_batch = [], None
+    for s_, T in ((sa, A), (sb, B)):
+        k = momentum_of(T)
+        if k is None or len(k.axes) != T.dim() or T.dim() != len(s_):
+            return None
+        if r not in s_:
+            sliced.append((s_, T, 0))
+            continue
+        d = s_.index(r)
+        if k.axes[d][2] != 0 or int(T.shape[d]) < 1 or (n_batch is not None and n_batch != int(T.shape[d])):
+            return None
+        n_batch = int(T.shape[d])
+        v = T.select(d, 0)
+        _set_momentum(v, k.with_axes(k.axes[:d] + k.axes[d + 1:]))
+        sliced.append((s_.replace(r, ""), v, int(T.stride(d))))
+    (sa1, A1, a_bstr), (sb1, B1, b_bstr) = sliced
+    g = _group_term(out_sub[1:], (alpha, sa1, A1, sb1, B1))
+    if g is None:
+        return None
+    return float(alpha), sa, A, sb, B, g, n_batch, a_bstr, b_bstr
+
+
+def _run_group_batched(out_sub, t, out, beta):
+    """One term of :func:`_batched_group_term` through ``pmb_group_contract_batched``: the group
+    plan of one right-hand side serves all of them (planned once per geometry, whatever the batch
+    size).  Elements outside every group are cleared (beta = 0) or scaled (beta != 1) here."""
+    _alpha, sa, _A, sb, _B, g, n_batch, a_bstr, b_bstr = t
+    c_bstr = int(out.stride(0))
+    plan = _group_plan(out_sub[1:], g, out.select(0, 0))
+    if beta == 0.0:
+        out.zero_()
+    elif beta != 1.0:
+        for k in range(out.shape[0]):
+            axpby(beta, out[k], 0.0, out[k])
+    d = _lib.GroupBatched()
+    d.n_batch, d.a_bstr, d.b_bstr, d.c_bstr = n_batch, a_bstr, b_bstr, c_bstr
+    if not plan["n_tiles"]:
+        _lib.check(_lib.load().pmb_group_contract_batched(C.byref(d), _stream()), "pmb_group_contract_batched")
+        return
+    alpha, _sa1, A1, _sb1, B1, _sigma = g
+    p = d.g
+    p.A, p.B, p.C = A1.data_ptr(), B1.data_ptr(), out.data_ptr()
+    p.a_row, p.a_ent, p.b_ent = plan["a_row"].data_ptr(), plan["a_ent"].data_ptr(), plan["b_ent"].data_ptr()
+    p.b_col, p.c_row, p.c_col = plan["b_col"].data_ptr(), plan["c_row"].data_ptr(), plan["c_col"].data_ptr()
+    p.tiles, p.n_tiles, p.alpha = plan["tiles"].data_ptr(), int(plan["n_tiles"]), alpha
+    trace = _timing["trace"]
+    if trace is not None:
+        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        t0.record(torch.cuda.current_stream())
+    rc = _lib.load().pmb_group_contract_batched(C.byref(d), _stream())
+    if trace is not None:
+        t1.record(torch.cuda.current_stream())
+        trace.append(("%s,%s->%s [momentum-blocked x%d]" % (sa, sb, out_sub, n_batch), plan["flops"] * n_batch,
+                      t0, t1))
+    _lib.check(rc, "pmb_group_contract_batched")
+
+
 def _try_blocked(out_sub, terms, out, beta):
     """Terms with momentum structure are evaluated on their diagonal blocks only: both operands
-    with a live momentum rule by ``pmb_group_contract`` (``_group_term``), a
+    with a live momentum rule by ``pmb_group_contract`` (``_group_term``; repeated over stacked
+    right-hand sides by ``pmb_group_contract_batched``, ``_batched_group_term``), a
     stored or generated integral block times a dense operand by ``pmb_blocked_contract``
     (``_blocked_term``).  The other terms of the same call (e.g. the hole-hole ladder next to the
     particle-particle one, ccd.py:185-187) keep the dense kernel.  Returns the result, or None when
     no term qualifies."""
     picked = []
     for i, t in enumerate(terms):
+        bt = _batched_group_term(out_sub, t)
+        if bt is not None:
+            picked.append((i, "batched", bt))
+            continue
         g = _group_term(out_sub, t)
         if g is not None:
             picked.append((i, "group", g))
@@ -1182,7 +1278,9 @@ def _try_blocked(out_sub, terms, out, beta):
         contract_terms(out_sub, rest, out=out, beta=beta)
         beta = 1.0
     for i, kind, t in picked:
-        if kind == "group":
+        if kind == "batched":
+            _run_group_batched(out_sub, t, out, beta)
+        elif kind == "group":
             _run_group(out_sub, t, out, beta)
         elif not _run_blocked(out_sub, t, out, beta):
             continue
@@ -1224,7 +1322,7 @@ def _contract_terms(out_sub, terms, out, beta):
                            "(there is no CPU fallback)" % (out.device, device()))
     # a term whose operands both carry a live rule runs on its momentum groups, however cheap the
     # matrix-vector or gather kernel would be: the group plan skips every product the rules make zero
-    if any(_group_term(out_sub, t) is not None for t in terms):
+    if any(_group_term(out_sub, t) is not None or _batched_group_term(out_sub, t) is not None for t in terms):
         return _try_blocked(out_sub, terms, out, beta)
     res = _try_gemv(out_sub, terms, out, beta)
     if res is not None:
@@ -1400,6 +1498,35 @@ def sym_baji(Ex, R=None, accumulate=True):
     _lib.check(lib.pmb_sym_baji(no, nv, _ptr(Ex), _ptr(R), int(accumulate), _stream()), "pmb_sym_baji")
     _written(R, k, chain)
     return R
+
+
+def sym_baji_stack(Ex, R):
+    """R[k] = Ex[k] + Ex[k]^{baji} for every k of the stacks Ex, R [r,v,v,o,o] (``sym_baji`` per
+    right-hand side); R keeps the rule of Ex when the swap leaves it unchanged."""
+    k, chain = momentum_of(Ex), _chain(R)
+    if k is not None and k.permute((0, 2, 1, 4, 3)) != k:
+        k = None
+    for i in range(Ex.shape[0]):
+        sym_baji(Ex[i], R[i], accumulate=False)
+    _written(R, k, chain)
+    return R
+
+
+def stack(tensors):
+    """``torch.stack`` along a new leading axis; the result keeps the rule the inputs share (the new
+    axis, a batch of right-hand sides, gets sign 0), none when they do not all carry the same one."""
+    keys = {momentum_of(t) for t in tensors}
+    out = torch.stack(list(tensors))
+    key = keys.pop() if len(keys) == 1 else None
+    _set_momentum(out, key.with_axes([(0, len(tensors), 0)] + list(key.axes)) if key is not None else None)
+    return out
+
+
+def clear(t, rule=None):
+    """Zero ``t`` in place and tag it with ``rule`` (zeros satisfy any rule); returns ``t``."""
+    t.zero_()
+    _set_momentum(t, rule)
+    return t
 
 
 def _ptr_array(tensors):

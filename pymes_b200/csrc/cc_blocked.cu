@@ -303,7 +303,10 @@ constexpr int GT = 32, GK = 32, GNT = 256, GE = 4;
 static_assert(GE * GNT <= GK * (GT + 1), "the entry-split partial sums reuse As");
 static_assert((GNT & (GNT - 1)) == 0, "tree reduction over GNT threads");
 
-__global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_group_t p) {
+// One tile of a group product.  A, B and C are the operands of one right-hand side: the batched
+// entry point offsets the descriptor's pointers by its batch strides.
+__device__ __forceinline__ void group_tile(const pmb_group_t &p, const double *A, const double *B,
+                                           double *C) {
     __shared__ double As[GK][GT + 1];
     __shared__ double Bs[GK][GT + 1];
     __shared__ long long s_ar[GT], s_cr[GT], s_bc[GT], s_cc[GT];
@@ -330,7 +333,7 @@ __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_
             const long long ae = __ldg(p.a_ent + e0 + k), be = __ldg(p.b_ent + e0 + k);
 #pragma unroll
             for (int o = 0; o < GE; ++o)
-                if (o < no) acc[o] = fma(__ldg(p.A + s_ar[o / cn] + ae), __ldg(p.B + be + s_bc[o % cn]), acc[o]);
+                if (o < no) acc[o] = fma(__ldg(A + s_ar[o / cn] + ae), __ldg(B + be + s_bc[o % cn]), acc[o]);
         }
         double *red = &As[0][0];                  // [GE][GNT]
 #pragma unroll
@@ -343,7 +346,7 @@ __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_
             }
         }
         __syncthreads();
-        if (tid < no) p.C[s_cr[tid / cn] + s_cc[tid % cn]] += p.alpha * red[tid * GNT];
+        if (tid < no) C[s_cr[tid / cn] + s_cc[tid % cn]] += p.alpha * red[tid * GNT];
         return;
     }
     const int tx = tid % 16, ty = tid / 16;       // columns tx, tx+16; rows ty, ty+16
@@ -355,8 +358,8 @@ __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_
             const bool kok = kc + k < en;
             const long long ae = kok ? __ldg(p.a_ent + e0 + kc + k) : 0;
             const long long be = kok ? __ldg(p.b_ent + e0 + kc + k) : 0;
-            As[k][m] = (kok && m < rn) ? __ldg(p.A + s_ar[m] + ae) : 0.0;
-            Bs[k][m] = (kok && m < cn) ? __ldg(p.B + be + s_bc[m]) : 0.0;
+            As[k][m] = (kok && m < rn) ? __ldg(A + s_ar[m] + ae) : 0.0;
+            Bs[k][m] = (kok && m < cn) ? __ldg(B + be + s_bc[m]) : 0.0;
         }
         __syncthreads();
 #pragma unroll 8
@@ -378,10 +381,20 @@ __global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_
         for (int j = 0; j < 2; ++j) {
             const int n = tx + 16 * j;
             if (n >= cn) continue;
-            double *c = p.C + s_cr[m] + s_cc[n];
+            double *c = C + s_cr[m] + s_cc[n];
             *c += p.alpha * acc[i][j];
         }
     }
+}
+
+__global__ void __launch_bounds__(GNT) group_kernel(const __grid_constant__ pmb_group_t p) {
+    group_tile(p, p.A, p.B, p.C);
+}
+
+// blockIdx.y = right-hand side; a batch stride of 0 shares that operand between all of them
+__global__ void __launch_bounds__(GNT) group_batched_kernel(const __grid_constant__ pmb_group_batched_t p) {
+    const long long b = blockIdx.y;
+    group_tile(p.g, p.g.A + b * p.a_bstr, p.g.B + b * p.b_bstr, p.g.C + b * p.c_bstr);
 }
 
 // One pass over a strided tensor: max |x| where the signed momenta of its indices do not cancel.
@@ -432,6 +445,19 @@ extern "C" int pmb_group_contract(const pmb_group_t *d, pmb_stream_t stream) {
         !d->c_col || !d->tiles)
         return PMB_E_BADARG;
     group_kernel<<<(unsigned)d->n_tiles, GNT, 0, (cudaStream_t)stream>>>(*d);
+    count_launch();
+    return cuda_status();
+}
+
+extern "C" int pmb_group_contract_batched(const pmb_group_batched_t *d, pmb_stream_t stream) {
+    if (!d || d->g.n_tiles < 0 || d->n_batch < 1 || d->n_batch > 65535) return PMB_E_BADARG;
+    // each right-hand side owns its outputs: a C shared by several would be summed into twice
+    if (d->c_bstr == 0 && d->n_batch > 1) return PMB_E_BADARG;
+    if (d->g.n_tiles == 0) return 0;
+    const pmb_group_t &g = d->g;
+    if (!g.A || !g.B || !g.C || !g.a_row || !g.a_ent || !g.b_ent || !g.b_col || !g.c_row || !g.c_col || !g.tiles)
+        return PMB_E_BADARG;
+    group_batched_kernel<<<dim3((unsigned)g.n_tiles, (unsigned)d->n_batch), GNT, 0, (cudaStream_t)stream>>>(*d);
     count_launch();
     return cuda_status();
 }

@@ -574,6 +574,99 @@ def linear_momenta(model):
     return lin
 
 
+class ExcitationSector:
+    """One total-momentum sector of the excitations of a UEG reference: the singles a <- i with
+    l(k_a) - l(k_i) = l(K) and the doubles ab <- ij with l(k_a) + l(k_b) - l(k_i) - l(k_j) = l(K).
+    Made by :func:`excitation_sector`; it hands out the momentum rules (``backend.Momentum``) of
+    the tensors an EOM solve in the sector meets, so that the solver never sees the linearised
+    labels themselves."""
+
+    def __init__(self, lin, no, label, K=None):
+        self.lin, self.no, self.label = lin, int(no), int(label)
+        self.nv = len(lin) - self.no
+        self.K = None if K is None else tuple(int(x) for x in K)
+
+    def __repr__(self):
+        return "ExcitationSector(K=%s, l(K)=%d)" % (self.K, self.label)
+
+    def __eq__(self, other):
+        return isinstance(other, ExcitationSector) and self.no == other.no and self.label == other.label \
+            and np.array_equal(self.lin, other.lin)
+
+    def __hash__(self):
+        return hash((self.no, self.label, len(self.lin)))
+
+    def rule(self, key, total=0):
+        """Rule of a tensor indexed like ``key`` (occupied letters i-l, virtual a-h; two indices
+        signed (+,-), four (+,+,-,-), the integral blocks' <pq|rs> convention) with ``total``."""
+        if len(key) not in (2, 4):
+            raise ValueError("a rule for 2 or 4 indices, not %r" % key)
+        signs = (1, -1) if len(key) == 2 else SIGNS
+        axes = [((0, self.no) if ch in "ijkl" else (self.no, self.nv)) + (sg,) for ch, sg in zip(key, signs)]
+        return bk.Momentum(self.lin, axes, total=total)
+
+    def fock_rule(self):
+        """Rule of the (dressed) Fock matrix over all orbitals: momentum-diagonal."""
+        n = self.no + self.nv
+        return bk.Momentum(self.lin, [(0, n, 1), (0, n, -1)])
+
+    def singles_rule(self):
+        return self.rule("ai", self.label)
+
+    def doubles_rule(self):
+        return self.rule("abij", self.label)
+
+    def singles_mask(self):
+        """[v, o] booleans: the singles of the sector."""
+        lo, lv = self.lin[:self.no], self.lin[self.no:]
+        return (lv[:, None] - lo[None, :]) == self.label
+
+
+def excitation_sector(model, no, K):
+    """The sector of total momentum ``K`` (an integer 3-vector, in units of the reciprocal lattice of
+    the box) of the excitations of ``model`` with ``no`` occupied orbitals.
+
+    The sector is defined by the LINEAR label l(K) = n^2 K_x + n K_y + K_z, n = 2 imax + 1, and not
+    by the vector K: that label is what the reference's integrals conserve, including the aliased
+    elements described in :func:`momentum_groups` (a component beyond imax carries into the next
+    digit).  H-bar built from them therefore couples exactly the excitations with equal l(K).  Where
+    two different vectors K and K' have l(K) = l(K') -- a difference k_a - k_i has components up to
+    2 imax, so it can -- they are ONE sector here, and its states are not sorted by vector K."""
+    K = np.asarray(K)
+    if K.shape != (3,) or not np.issubdtype(K.dtype, np.integer):
+        raise ValueError("K must be an integer 3-vector")
+    n = 2 * int(model.imax) + 1
+    label = n * n * int(K[0]) + n * int(K[1]) + int(K[2])
+    return ExcitationSector(linear_momenta(model), no, label, K)
+
+
+def excitation_sectors(model, no):
+    """Every sector that holds at least one single (a, i): a list of dicts ``{"K", "sector",
+    "n_singles", "n_doubles", "aliases"}`` sorted by |K| (then by K).  ``K`` is the shortest
+    k_a - k_i of the sector; ``aliases`` lists the other vectors k_a - k_i with the same linear label
+    (see :func:`excitation_sector`)."""
+    k = model.k_int().astype(np.int64)
+    lin = linear_momenta(model)
+    lo, lv = lin[:no], lin[no:]
+    dk = (k[no:][:, None, :] - k[:no][None, :, :]).reshape(-1, 3)
+    lab = (lv[:, None] - lo[None, :]).reshape(-1)
+    # doubles per label: histogram of l_a + l_b against that of l_i + l_j
+    pv, cv = np.unique(np.add.outer(lv, lv).reshape(-1), return_counts=True)
+    po, co = np.unique(np.add.outer(lo, lo).reshape(-1), return_counts=True)
+    out = []
+    for l_ in np.unique(lab):
+        vecs = np.unique(dk[lab == l_], axis=0)
+        vecs = vecs[np.lexsort((vecs[:, 2], vecs[:, 1], vecs[:, 0], (vecs ** 2).sum(axis=1)))]
+        want = po + l_
+        hit = np.isin(want, pv)
+        n_dbl = int((co[hit] * cv[np.searchsorted(pv, want[hit])]).sum())
+        out.append({"K": tuple(int(x) for x in vecs[0]), "aliases": [tuple(int(x) for x in v) for v in vecs[1:]],
+                    "sector": ExcitationSector(lin, no, int(l_), vecs[0]), "n_singles": int((lab == l_).sum()),
+                    "n_doubles": n_dbl})
+    out.sort(key=lambda e: (sum(x * x for x in e["K"]), e["K"]))
+    return out
+
+
 def momentum_rule(model, lo, ext, signs=SIGNS):
     """``backend.Momentum`` of a tensor over the orbital ranges ``lo`` / ``ext`` with the given signs
     (an integral block: (+,+,-,-); the Fock matrix: (+,-))."""

@@ -276,6 +276,15 @@ class DressedLadder(bk.LinearOperator):
         bk.bdot("bl,lab->ab", T1, Z, out=D, alpha=1.0, beta=1.0)
         return D
 
+    def adopt_momentum(self, rule_of):
+        """Check (and tag) the operator's parts under their momentum rules ``rule_of(key)`` (key:
+        "abcd", "iabc", "aibc", "ijab", "ai"); True when every part conserves momentum."""
+        V = self.V_abcd
+        ok = V.momentum() == rule_of("abcd") if isinstance(V, bk.GeneratedOperand) else \
+            bk.adopt_momentum(V, rule_of("abcd"))
+        return ok and all(bk.adopt_momentum(t, rule_of(k)) for k, t in
+                          (("iabc", self.V_iabc), ("aibc", self.V_aibc), ("ijab", self.V_ijab), ("ai", self.T1)))
+
     def dense(self):
         """The dressed block itself (tests / small systems)."""
         V = self.V_abcd.materialise() if isinstance(self.V_abcd, bk.GeneratedOperand) else self.V_abcd

@@ -108,7 +108,10 @@ class SigmaPlan:
         self.no = no
         self.shard = shard
         self.nv = nv = T2.shape[0]
-        self.static = {"foo": fock[:no, :no], "fov": fock[:no, no:], "fvv": fock[no:, no:], "T": T2}
+        # bk.narrow: the blocks keep the Fock matrix's momentum rule (a sector's products need it)
+        rows_o, rows_v = bk.narrow(fock, 0, 0, no), bk.narrow(fock, 0, no, nv)
+        self.static = {"foo": bk.narrow(rows_o, 1, 0, no), "fov": bk.narrow(rows_o, 1, no, nv),
+                       "fvv": bk.narrow(rows_v, 1, no, nv), "T": T2}
         for key in V_KEYS_USED:
             self.static[key] = dV[key]
         # a hoisted intermediate may be as large as one o.v^3 integral block
@@ -199,11 +202,12 @@ class SigmaPlan:
         """(alpha, W): a zero-copy permuted view when the group is one plain operand, otherwise
         the coefficient-weighted sum of the group's operands / hoisted products.  In a sharded
         plan a W that carries the output index ``a`` is built for this rank's rows only (the
-        hoisted products are the big replicated memory otherwise: up to o.v^3 each)."""
+        hoisted products are the big replicated memory otherwise: up to o.v^3 each).  The first
+        item is written, not accumulated, so that W carries the momentum rule its items derive."""
         rows = self._rows
         if len(items) == 1 and len(items[0][1]) == 1:
             coef, [(s, n)] = items[0]
-            return coef, rows(wsub, self.static[n].permute(*[s.index(ch) for ch in wsub]))
+            return coef, rows(wsub, bk.permute(self.static[n], [s.index(ch) for ch in wsub]))
         ext = {}
         for _, stat in items:
             for s, n in stat:
@@ -211,15 +215,17 @@ class SigmaPlan:
                     ext[ch] = int(e)
         if self.shard is not None and "a" in wsub:
             ext["a"] = self.shard.na
-        W = bk.zeros(*[ext[ch] for ch in wsub])
+        W = bk.empty(*[ext[ch] for ch in wsub])
+        beta = 0.0
         for coef, stat in items:
             if len(stat) == 1:
                 s, n = stat[0]
-                bk.axpby(coef, rows(wsub, self.static[n].permute(*[s.index(ch) for ch in wsub])), 1.0, W)
+                bk.axpby(coef, rows(wsub, bk.permute(self.static[n], [s.index(ch) for ch in wsub])), beta, W)
             else:
                 (s1, n1), (s2, n2) = stat
                 bk.contract_terms(wsub, [(coef, s1, rows(s1, self.static[n1]), s2, rows(s2, self.static[n2]))],
-                                  out=W, beta=1.0)
+                                  out=W, beta=beta)
+            beta = 1.0
         return 1.0, W
 
     # ---- execution -----------------------------------------------------
@@ -251,22 +257,22 @@ class SigmaPlan:
 
     def apply(self, U1, U2, out=None):
         """sigma for a batch: U1 [r,v,o], U2 [r,v,v,o,o] device tensors (any strides along r,
-        each vector contiguous) -> (S1, S2).  eom_ccsd.py:268-385 for every r at once."""
+        each vector contiguous) -> (S1, S2).  eom_ccsd.py:268-385 for every r at once.  Stacks
+        with a momentum rule (``bk.stack`` of sector vectors) run every product on momentum groups
+        and give S1, S2 with the same rules."""
         U = {"u1": U1, "u2": U2}
         r = U2.shape[0]
         if self.shard is not None:
             return self._apply_sharded(U, r, out)
         if out is None:
-            S1, S2 = bk.zeros(*U1.shape), bk.empty(*U2.shape)
+            S1, S2 = bk.zeros(*U1.shape, rule=bk.momentum_of(U1)), bk.empty(*U2.shape)
         else:
             S1, S2 = out
-            for k in range(r):
-                S1[k].zero_()
+            bk.clear(S1, bk.momentum_of(U1))
         self._run(self.programs["s1"], U, S1)
-        Ex = bk.zeros(*U2.shape)
+        Ex = bk.zeros(*U2.shape, rule=bk.momentum_of(U2))
         self._run(self.programs["s2p"], U, Ex)
-        for k in range(r):                                             # eom_ccsd.py:377
-            bk.sym_baji(Ex[k], S2[k], accumulate=False)
+        bk.sym_baji_stack(Ex, S2)                                      # eom_ccsd.py:377
         del Ex
         self._run(self.programs["s2n"], U, S2)
         return S1, S2
@@ -399,15 +405,28 @@ def _as_dict_dev(dict_t_V):
 
 
 class EOM_CCSD:
-    def __init__(self, no, n_excit=3, comm=None, parallel="rows"):
+    def __init__(self, no, n_excit=3, comm=None, parallel="rows", sector=None):
         """``comm`` (extension, ``pymes_b200.parallel.Comm``) with ``parallel="rows"``: the sigma
         product is evaluated in (ab) row blocks over the ranks of ``comm`` (operators too large
         for one GPU); with ``parallel="vectors"``: every rank holds the full operator and applies
         it to its share of each batch of new trial vectors, the results are summed over the ranks
         (no exchange inside sigma).  Everything else (trial vectors, the projected eigenproblem) is
-        replicated and identical on every rank."""
+        replicated and identical on every rank.
+
+        ``sector`` (extension, ``model.ueg.excitation_sector``): :meth:`solve` finds the lowest
+        states of ONE total momentum of a UEG reference.  H-bar built from momentum-conserving
+        integrals never mixes sectors, so the Davidson space is kept inside the sector: the guesses
+        are the sector's lowest singles, and every new trial vector is checked to lie in it (one
+        pass per vector; a vector with weight outside raises) before sigma sees it, which then runs
+        every product that involves it on momentum groups.  The dressed Fock matrix, T2 and the
+        integral blocks are checked to conserve momentum when the sigma program is built
+        (``ValueError`` if one does not: the sector would not be invariant).  Vectors keep the dense
+        [v,o] / [v,v,o,o] layout.  Not available together with a sector: a ``comm`` of more than one
+        rank and ``preconditioner = "diagonal"`` (both raise ``NotImplementedError``)."""
         if parallel not in ("rows", "vectors"):
             raise ValueError("parallel must be 'rows' or 'vectors'")
+        if sector is not None and comm is not None and comm.size > 1:
+            raise NotImplementedError("EOM-CCSD in a momentum sector runs on one device (no comm)")
         self.algo_name = "EOM-CCSD"
         # "scalar": the reference's correction vectors, r / (e_n - D_guess_n + 1e-5) with ONE number per
         # root (eom_ccsd.py:140-141).  "diagonal" (extension, not the reference's iterates): the usual
@@ -427,6 +446,7 @@ class EOM_CCSD:
         self.max_iter = 500
         self._plan = None
         self._plan_key = None
+        self.sector = sector
 
     def write_logging_info(self):
         return
@@ -449,14 +469,34 @@ class EOM_CCSD:
         key = (self._ident(t_fock_pq), id(dict_t_V), self._ident(t_T_abij))
         if self._plan is None or self._plan_key != key:
             T2 = bk.asdev(t_T_abij).contiguous()
+            fock, dV = bk.asdev(t_fock_pq), _as_dict_dev(dict_t_V)
             shard = None
-            if self.comm is not None and self.comm.size > 1:
+            if self.sector is not None:
+                self._adopt_operands(t_fock_pq, fock, dV, T2)
+            elif self.comm is not None and self.comm.size > 1:
                 from ..parallel import Shard
                 shard = Shard(self.comm, T2.shape[0])
-            self._plan = SigmaPlan(self.no, bk.asdev(t_fock_pq), _as_dict_dev(dict_t_V), T2, shard=shard)
+            self._plan = SigmaPlan(self.no, fock, dV, T2, shard=shard)
             self._plan_key = key
             self._keep = (t_fock_pq, dict_t_V, t_T_abij)        # keep ids alive
         return self._plan
+
+    def _adopt_operands(self, t_fock_pq, fock, dV, T2):
+        """Tag the operands of a sector's sigma with their (total 0) momentum rules, after checking
+        that every element a rule forbids is zero; ``ValueError`` names the first that breaks it."""
+        sec = self.sector
+        host = None if isinstance(t_fock_pq, torch.Tensor) else np.asarray(t_fock_pq)
+        checks = [("the Fock matrix", bk.adopt_momentum(fock, sec.fock_rule(), host=host)),
+                  ("T2", bk.adopt_momentum(T2, sec.rule("abij")))]
+        for k in V_KEYS_USED:
+            if isinstance(dV[k], bk.LinearOperator):
+                checks.append(("V_" + k, dV[k].adopt_momentum(sec.rule)))
+            else:
+                checks.append(("V_" + k, bk.adopt_momentum(dV[k], sec.rule(k))))
+        for what, ok in checks:
+            if not ok:
+                raise ValueError("%s does not conserve momentum: H-bar would mix the sector %r with others"
+                                 % (what, sec))
 
     def sigma_batched(self, t_fock_pq, dict_t_V, U1, U2, t_T_abij):
         """(H-bar U)_singles, (H-bar U)_doubles for stacked vectors U1 [r,v,o], U2 [r,v,v,o,o]."""
@@ -507,7 +547,7 @@ class EOM_CCSD:
         S2 = bk.zeros(n, nv, nv, no, no) if vc is not None else bk.empty(n, nv, nv, no, no)
         for b0 in range(lo, hi, self.max_rhs):
             b1 = min(b0 + self.max_rhs, hi)
-            plan.apply(torch.stack(u1s[b0:b1]), torch.stack(u2s[b0:b1]), out=(S1[b0:b1], S2[b0:b1]))
+            plan.apply(bk.stack(u1s[b0:b1]), bk.stack(u2s[b0:b1]), out=(S1[b0:b1], S2[b0:b1]))
         if vc is not None:
             vc.all_reduce_sum(S1)
             vc.all_reduce_sum(S2)
@@ -548,7 +588,19 @@ class EOM_CCSD:
         nv = T2.shape[0]
         fd = bk.tonumpy(fock).diagonal()
         D_ai = -(fd[:no][None, :] - fd[no:][:, None]).ravel()
-        lowest = np.argsort(D_ai)[:n_excit]
+        sec = self.sector
+        if sec is None:
+            lowest = np.argsort(D_ai)[:n_excit]
+        else:
+            if self.preconditioner != "scalar":
+                raise NotImplementedError("EOM-CCSD in a momentum sector uses the scalar preconditioner")
+            inside = sec.singles_mask().ravel()
+            if not inside.any():
+                raise ValueError("the sector %r holds no single excitation" % (sec,))
+            if n_excit > inside.sum():
+                raise ValueError("n_excit = %d exceeds the %d singles of the sector %r" % (n_excit, inside.sum(), sec))
+            lowest = np.argsort(np.where(inside, D_ai, np.inf))[:n_excit]
+            rule1, rule2 = sec.singles_rule(), sec.doubles_rule()
         plan = self.plan(t_fock_dressed_pq, dict_t_V_dressed, t_T_abij)
 
         print_logging_info("Initialising u tensors...", level=1)
@@ -575,6 +627,10 @@ class EOM_CCSD:
             m = len(u1s)
             n_done = len(w1s)
             u1s, u2s = orthonormalise(u1s, u2s, start=n_done)
+            if sec is not None:
+                for n in range(n_done, m):
+                    if not (bk.adopt_momentum(u1s[n], rule1) and bk.adopt_momentum(u2s[n], rule2)):
+                        raise RuntimeError("trial vector %d has weight outside the sector %r" % (n, sec))
             if n_done < m:
                 S1, S2 = self.sigma_list(plan, u1s[n_done:], u2s[n_done:])
                 w1s += S1
