@@ -102,14 +102,22 @@ typedef struct {
 
 /* bytes of scratch needed for `d` (split-K partial sums; 0 if not split)    */
 size_t pmb_contract_workspace(const pmb_contract_t *d);
+/* Terms with alpha = 0 contribute nothing and are skipped.  The other terms   */
+/* are issued in runs of consecutive terms whose |alpha| lie within a factor   */
+/* 2^64 of each other (every term of ordinary coefficients: one run); each run */
+/* is one launch sequence, the caller's beta on the first, beta = 1 after it,  */
+/* so coefficients as far apart as 2^600 and 2^-600 neither overflow nor       */
+/* underflow.  The workspace is the largest any run needs.                    */
 int pmb_contract(const pmb_contract_t *d, void *ws, size_t ws_bytes,
                  pmb_stream_t stream);
 /* tuning/diagnostic knobs: force a tile configuration (-1 = heuristic; bits   */
 /* 0-2 the configuration, +8 flips the copy interleaving, +16 makes generated  */
 /* operands use the scanning producer instead of the non-zero walker, +32 keeps */
-/* the n-fastest tile order for launches with a generated operand, +256 keeps   */
-/* it for stored operands too instead of the banded order) and                 */
-/* a split-K factor (0 = heuristic).                                          */
+/* the n-fastest tile order for launches with a generated operand, +64 keeps    */
+/* the sparse last wave of the warp-specialised kernel instead of splitting it */
+/* over k, +128 copies B 8 bytes at a time where 16-byte copies are possible,  */
+/* +256 keeps the n-fastest order for stored operands too instead of the       */
+/* banded order) and a split-K factor (0 = heuristic).                        */
 void pmb_contract_set_tuning(int tile_config, int split_k);
 /* L2 budget (bytes) for one operand's k window; contractions whose smaller      */
 /* operand exceeds it are issued as a fixed-order sequence of k-window launches */

@@ -25,6 +25,7 @@
 // thread->element mapping of the gathers that follows each operand's
 // unit-stride direction (x-fast or k-fast) so global accesses stay coalesced
 // to full 32 B sectors for any permutation.
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 
@@ -1496,7 +1497,50 @@ extern "C" void pmb_contract_set_panel_bytes(long long bytes) {
     g_panel_bytes_ws = bytes < 0 ? kPanelDefaultWs : bytes;
 }
 
-extern "C" size_t pmb_contract_workspace(const pmb_contract_t *d) {
+namespace pmb {
+
+// Coefficient runs.  The kernels keep their accumulators in units of the current term's alpha and
+// rescale them by alpha_old / alpha_new at a term boundary, which overflows or underflows when the
+// coefficients are far apart (alphas 2^600 and 2^-600: the ratio is inf).  The terms are therefore
+// issued in runs of consecutive terms whose non-zero finite |alpha| lie within a factor 2^kCoefSpread
+// of each other -- one launch sequence per run, the caller's beta on the first, beta = 1 after it.
+// Ordinary coefficients form one run: one launch sequence, as before.
+constexpr int kCoefSpread = 64;
+
+// split the terms of `d` into runs: run r is terms [first[r], first[r + 1]); returns the count
+static int coef_runs(const pmb_contract_t *d, int *first) {
+    int nrun = 1, lo = 0, hi = 0;
+    bool open = false;
+    first[0] = 0;
+    for (int ti = 0; ti < d->nterms; ++ti) {
+        const double a = d->terms[ti].alpha;
+        if (a == 0.0 || !std::isfinite(a)) continue;      // dropped, or fits any run
+        const int e = std::ilogb(a);
+        if (!open) {
+            lo = hi = e;
+            open = true;
+        } else if ((e > hi ? e : hi) - (e < lo ? e : lo) > kCoefSpread) {
+            first[nrun++] = ti;
+            lo = hi = e;
+        } else {
+            lo = e < lo ? e : lo;
+            hi = e > hi ? e : hi;
+        }
+    }
+    first[nrun] = d->nterms;
+    return nrun;
+}
+
+// descriptor of run r: its terms, beta = 1 after the first run
+static pmb_contract_t run_descriptor(const pmb_contract_t *d, const int *first, int r) {
+    pmb_contract_t q = *d;
+    q.nterms = first[r + 1] - first[r];
+    for (int i = 0; i < q.nterms; ++i) q.terms[i] = d->terms[first[r] + i];
+    if (r > 0) q.beta = 1.0;
+    return q;
+}
+
+static size_t workspace_one(const pmb_contract_t *d) {
     Params p;
     int cfg;
     if (build_params(d, p, cfg) != 0) return 0;
@@ -1507,12 +1551,51 @@ extern "C" size_t pmb_contract_workspace(const pmb_contract_t *d) {
     return sizeof(double) * (size_t)p.nsplit * (size_t)p.M * (size_t)p.N;
 }
 
+static int contract_one(const pmb_contract_t *d, void *ws, size_t ws_bytes, cudaStream_t s);
+
+}  // namespace pmb
+
+extern "C" size_t pmb_contract_workspace(const pmb_contract_t *d) {
+    if (!d || d->nterms < 1 || d->nterms > PMB_MAX_TERMS) return 0;
+    int first[PMB_MAX_TERMS + 1];
+    const int nrun = coef_runs(d, first);
+    if (nrun == 1) return workspace_one(d);
+    Params p;
+    int cfg;
+    if (build_params(d, p, cfg) != 0) return 0;
+    size_t need = 0;
+    for (int r = 0; r < nrun; ++r) {
+        const pmb_contract_t q = run_descriptor(d, first, r);
+        const size_t w = workspace_one(&q);
+        need = w > need ? w : need;
+    }
+    return need;
+}
+
 extern "C" int pmb_contract(const pmb_contract_t *d, void *ws, size_t ws_bytes, pmb_stream_t stream) {
+    if (!d || d->nterms < 1 || d->nterms > PMB_MAX_TERMS) return PMB_E_BADARG;
+    int first[PMB_MAX_TERMS + 1];
+    const int nrun = coef_runs(d, first);
+    if (nrun == 1) return contract_one(d, ws, ws_bytes, (cudaStream_t)stream);
+    Params p;
+    int cfg;
+    const int rc = build_params(d, p, cfg);     // every argument error before anything launches
+    if (rc != 0) return rc;
+    const size_t need = pmb_contract_workspace(d);
+    if (need && (!ws || ws_bytes < need)) return PMB_E_WORKSPACE;
+    for (int r = 0; r < nrun; ++r) {
+        const pmb_contract_t q = run_descriptor(d, first, r);
+        const int rr = contract_one(&q, ws, ws_bytes, (cudaStream_t)stream);
+        if (rr != 0) return rr;
+    }
+    return 0;
+}
+
+int pmb::contract_one(const pmb_contract_t *d, void *ws, size_t ws_bytes, cudaStream_t s) {
     Params p;
     int cfg;
     int rc = build_params(d, p, cfg);
     if (rc != 0) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
     if (p.nsplit > 1) {
         const size_t need = sizeof(double) * (size_t)p.nsplit * (size_t)p.M * (size_t)p.N;
         if (!ws || ws_bytes < need) return PMB_E_WORKSPACE;

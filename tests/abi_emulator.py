@@ -417,15 +417,13 @@ class FakeLib:
             nz = _window(g.nz, ext[0] * ext[1] * ext[2]).reshape(ext[:3])
             blk = np.zeros(ext)
             n = 2 * u.imax + 1
-            for p in range(ext[0]):
-                for q in range(ext[1]):
-                    for r in range(ext[2]):
-                        v = kvec[lo[1] + q] - (kvec[lo[2] + r] - kvec[lo[0] + p]) + u.imax
-                        loc = n * n * v[0] + n * v[1] + v[2]
-                        if 0 <= loc < n ** 3 and lo[3] <= imap[loc] < lo[3] + ext[3]:
-                            blk[p, q, r, imap[loc] - lo[3]] = nz[p, q, r]
-                        else:
-                            assert nz[p, q, r] == 0.0
+            p, q, r = np.meshgrid(*[np.arange(e) for e in ext[:3]], indexing="ij")
+            v = kvec[lo[1] + q] - (kvec[lo[2] + r] - kvec[lo[0] + p]) + u.imax
+            loc = n * n * v[..., 0] + n * v[..., 1] + v[..., 2]
+            s = np.where((loc >= 0) & (loc < n ** 3), imap[np.clip(loc, 0, n ** 3 - 1)], -1)
+            hit = (s >= lo[3]) & (s < lo[3] + ext[3])
+            assert (nz[~hit] == 0.0).all()
+            blk[p[hit], q[hit], r[hit], s[hit] - lo[3]] = nz[hit]
         else:
             blk = self._block(g.ueg, g.W0a, g.W1a, g.W0s, lo, ext)
         nm = len(m_ext)
