@@ -243,6 +243,20 @@ int pmb_cdiv_shifted(int64_t n, const double *diag, double zr, double zi, double
                      const double *xr, const double *xi, double *yr, double *yi,
                      pmb_stream_t stream);
 
+/* Compact <-> dense vectors of one total-momentum sector (FEAST in a sector    */
+/* keeps only the allowed elements of its Krylov vectors), for right-hand      */
+/* sides 0 <= b < n_batch and 0 <= k < n_idx:                                   */
+/*   gather : dst[b*dst_bstr + k]      = src[b*src_bstr + idx[k]]               */
+/*   scatter: dst[b*dst_bstr + idx[k]] = src[b*src_bstr + k]  (others kept)     */
+/* idx: strictly increasing int64 offsets on the device, shared by every        */
+/* right-hand side; src and dst do not overlap.  64-bit offsets, any n_batch;   */
+/* plain copies (values pass bit-exact).  PMB_E_BADARG for n_batch < 1,         */
+/* n_idx < 1 or a null pointer.                                                 */
+int pmb_sector_gather(int64_t n_batch, int64_t n_idx, const int64_t *idx, const double *src,
+                      int64_t src_bstr, double *dst, int64_t dst_bstr, pmb_stream_t stream);
+int pmb_sector_scatter(int64_t n_batch, int64_t n_idx, const int64_t *idx, const double *src,
+                       int64_t src_bstr, double *dst, int64_t dst_bstr, pmb_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* UEG momentum-conserving two-electron integrals  pymes/model/ueg.py:265-596 */
 /*                                                                          */

@@ -113,6 +113,10 @@ _SIGS = {
     "pmb_gemv": (C.c_int, [C.POINTER(Gemv), C.c_void_p]),
     "pmb_cdiv_shifted": (C.c_int, [C.c_int64, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pmb_sector_gather": (C.c_int, [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.c_int64, C.c_void_p]),
+    "pmb_sector_scatter": (C.c_int, [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                     C.c_int64, C.c_void_p]),
     "pmb_ueg_umat": (C.c_int, [C.POINTER(Ueg), C.c_double, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                C.c_void_p]),
     "pmb_ueg_pair_tables": (C.c_int, [C.POINTER(Ueg), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,

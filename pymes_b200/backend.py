@@ -1627,6 +1627,100 @@ def cdiv_shifted(diag, z, shift, xr, xi):
     return yr, yi
 
 
+def _sector_index(idx, row):
+    """Host copy of a sector index list ``idx`` (1-D contiguous int64 device tensor), checked once per
+    version of ``idx``: strictly increasing offsets inside a row of ``row`` elements."""
+    if not (isinstance(idx, torch.Tensor) and idx.dtype == torch.int64 and idx.dim() == 1 and idx.is_contiguous()):
+        raise ValueError("a sector index is a 1-D contiguous int64 tensor")
+    tag = getattr(idx, "_pmb_index", None)
+    if tag is None or tag[0] != idx._version:
+        h = idx.cpu().numpy()
+        if len(h) and (h[0] < 0 or np.any(np.diff(h) <= 0)):
+            raise ValueError("a sector index must be strictly increasing and non-negative")
+        tag = (idx._version, h, {})
+        idx._pmb_index = tag
+    h = tag[1]
+    if len(h) and h[-1] >= row:
+        raise ValueError("sector index %d is outside a row of %d elements" % (h[-1], row))
+    return tag
+
+
+def _sector_rows(t, batched, what):
+    """(n_batch, batch stride, row length) of a stack [r, ...] (``batched``) or one vector whose rows
+    are contiguous."""
+    if batched and (t.dim() < 2 or t.shape[0] < 1):
+        raise ValueError("%s: a stack [r, ...] of r >= 1 vectors" % what)
+    first = t[0] if batched else t
+    if not first.is_contiguous():
+        raise ValueError("%s: rows of a sector stack must be contiguous" % what)
+    return (t.shape[0] if batched else 1), (int(t.stride(0)) if batched else 0), first.numel()
+
+
+def sector_gather(x_packed_stack, idx, out=None):
+    """out[b, k] = x[b].flatten()[idx[k]]: the allowed elements of one momentum sector taken out of a
+    stack of dense vectors [r, ...] (each vector contiguous; ``pmb_sector_gather``).  ``out``: an
+    [r, len(idx)] tensor with contiguous rows (any row stride, e.g. columns of a wider compact stack),
+    allocated when None.  The result carries no rule."""
+    x = x_packed_stack
+    nb, xb, row = _sector_rows(x, True, "sector_gather")
+    _sector_index(idx, row)
+    n = idx.numel()
+    if out is None:
+        out = empty(nb, n)
+    if tuple(out.shape) != (nb, n) or out.stride(1) != 1:
+        raise ValueError("sector_gather: out must be [%d, %d] with contiguous rows" % (nb, n))
+    chain = _chain(out)
+    if n:
+        _lib.check(_lib.load().pmb_sector_gather(nb, n, _ptr(idx), _ptr(x), xb, _ptr(out), out.stride(0),
+                                                 _stream()), "pmb_sector_gather")
+    _written(out, None, chain)
+    return out
+
+
+def _index_fits(tag, key, shape):
+    """Whether every offset of a sector index lies where ``key`` allows a non-zero in a tensor of
+    ``shape`` (host check on the index alone, cached with it)."""
+    memo = tag[2]
+    if (key, shape) not in memo:
+        pos = np.unravel_index(tag[1], shape) if len(tag[1]) else [np.zeros(0, dtype=np.int64)] * len(shape)
+        tot = sum(key.labels(d)[p] for d, p in enumerate(pos))
+        memo[(key, shape)] = bool(np.all(tot == 0))
+    return memo[(key, shape)]
+
+
+def sector_scatter(compact, idx, out):
+    """out[b].flatten()[idx[k]] = compact[b, k] (``pmb_sector_scatter``); every other element of
+    ``out`` is left as it is.  ``compact`` [r, len(idx)] (or one vector [len(idx)]), ``out`` [r, ...]
+    (or one tensor), rows contiguous.  When ``out`` carried a live momentum rule before the write (a
+    ``zeros(..., rule=...)`` buffer) and every offset of ``idx`` is allowed by it, the write keeps
+    ``out`` inside the rule and ``out`` is re-stamped with it; otherwise ``out`` is left untagged."""
+    batched = compact.dim() == 2
+    if compact.dim() not in (1, 2) or compact.stride(-1) != 1:
+        raise ValueError("sector_scatter: compact must be [r, n] or [n] with contiguous rows")
+    nb, ob, row = _sector_rows(out, batched, "sector_scatter")
+    tag = _sector_index(idx, row)
+    n = idx.numel()
+    if tuple(compact.shape) != ((nb, n) if batched else (n,)):
+        raise ValueError("sector_scatter: compact of shape %s for %d vectors of %d elements"
+                         % (tuple(compact.shape), nb, n))
+    key, chain = momentum_of(out), _chain(out)
+    if key is not None:
+        shape = tuple(int(e) for e in out.shape)
+        if batched:                          # a stack: its batch axis must be unconstrained
+            key_row = key.with_axes(key.axes[1:]) if key.axes[0][2] == 0 else None
+            shape = shape[1:]
+        else:
+            key_row = key
+        if key_row is None or not _index_fits(tag, key_row, shape):
+            key = None
+    if n:
+        _lib.check(_lib.load().pmb_sector_scatter(nb, n, _ptr(idx), _ptr(compact),
+                                                  int(compact.stride(0)) if batched else 0, _ptr(out), ob,
+                                                  _stream()), "pmb_sector_scatter")
+    _written(out, key, chain)
+    return out
+
+
 def diag_view(t, sub, out_sub):
     """Strided VIEW of a tensor with repeated subscripts, e.g. diag_view(V, "iaai", "ai")[a,i] =
     V[i,a,a,i] (the einsum("iaai->ai") of eom_ccsd.py:182); no data is moved."""

@@ -486,3 +486,67 @@ extern "C" int pmb_momentum_residue(int ndim, const int64_t ext[4], const int64_
     count_launch();
     return cuda_status();
 }
+
+namespace pmb {
+namespace {
+
+// Compact <-> dense vectors of one momentum sector: right-hand side b copies n_idx doubles through
+// the index list idx (shared by every right-hand side).  Batches run over gridDim.y with a stride
+// loop, so any n_batch fits; offsets are 64-bit throughout.  Pure copies: values pass bit-exact.
+__global__ void __launch_bounds__(256)
+    sector_gather_kernel(int64_t n_batch, int64_t n_idx, const int64_t *__restrict__ idx,
+                         const double *__restrict__ src, int64_t src_bstr, double *__restrict__ dst,
+                         int64_t dst_bstr) {
+    for (int64_t b = blockIdx.y; b < n_batch; b += gridDim.y) {
+        const double *s = src + b * src_bstr;
+        double *d = dst + b * dst_bstr;
+        for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_idx;
+             k += (int64_t)gridDim.x * blockDim.x)
+            d[k] = s[idx[k]];
+    }
+}
+
+__global__ void __launch_bounds__(256)
+    sector_scatter_kernel(int64_t n_batch, int64_t n_idx, const int64_t *__restrict__ idx,
+                          const double *__restrict__ src, int64_t src_bstr, double *__restrict__ dst,
+                          int64_t dst_bstr) {
+    for (int64_t b = blockIdx.y; b < n_batch; b += gridDim.y) {
+        const double *s = src + b * src_bstr;
+        double *d = dst + b * dst_bstr;
+        for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_idx;
+             k += (int64_t)gridDim.x * blockDim.x)
+            d[idx[k]] = s[k];
+    }
+}
+
+// About 16 CTAs per SM in all: the index range first, the batch fills what it leaves.
+static dim3 sector_grid(int64_t n_batch, int64_t n_idx) {
+    long long bx = (n_idx + 255) / 256;
+    if (bx > 16LL * kSmCount) bx = 16LL * kSmCount;
+    long long by = (16LL * kSmCount) / bx;
+    if (by < 1) by = 1;
+    if (by > n_batch) by = n_batch;
+    if (by > 65535) by = 65535;
+    return dim3((unsigned)bx, (unsigned)by, 1);
+}
+
+}  // namespace
+}  // namespace pmb
+
+extern "C" int pmb_sector_gather(int64_t n_batch, int64_t n_idx, const int64_t *idx, const double *src,
+                                 int64_t src_bstr, double *dst, int64_t dst_bstr, pmb_stream_t stream) {
+    if (n_batch < 1 || n_idx < 1 || !idx || !src || !dst) return PMB_E_BADARG;
+    sector_gather_kernel<<<sector_grid(n_batch, n_idx), 256, 0, (cudaStream_t)stream>>>(
+        n_batch, n_idx, idx, src, src_bstr, dst, dst_bstr);
+    count_launch();
+    return cuda_status();
+}
+
+extern "C" int pmb_sector_scatter(int64_t n_batch, int64_t n_idx, const int64_t *idx, const double *src,
+                                  int64_t src_bstr, double *dst, int64_t dst_bstr, pmb_stream_t stream) {
+    if (n_batch < 1 || n_idx < 1 || !idx || !src || !dst) return PMB_E_BADARG;
+    sector_scatter_kernel<<<sector_grid(n_batch, n_idx), 256, 0, (cudaStream_t)stream>>>(
+        n_batch, n_idx, idx, src, src_bstr, dst, dst_bstr);
+    count_launch();
+    return cuda_status();
+}

@@ -621,6 +621,23 @@ class ExcitationSector:
         lo, lv = self.lin[:self.no], self.lin[self.no:]
         return (lv[:, None] - lo[None, :]) == self.label
 
+    def packed_index(self):
+        """Sorted int64 offsets of the sector's elements in the packed [singles | doubles] layout of
+        length v.o + v^2.o^2 (``SigmaPlan.apply_packed``): the singles a,i with l_a - l_i = l(K), then
+        v.o + the doubles a,b,i,j with l_a + l_b - l_i - l_j = l(K).  Built one virtual a at a time
+        (one [v, o^2] mask), cached on the sector."""
+        if getattr(self, "_packed", None) is None:
+            no, nv = self.no, self.nv
+            lo, lv = np.asarray(self.lin[:no], dtype=np.int64), np.asarray(self.lin[no:], dtype=np.int64)
+            n1, blk = nv * no, nv * no * no
+            lij = (lo[:, None] + lo[None, :]).reshape(-1)
+            parts = [np.flatnonzero(self.singles_mask())]
+            for a in range(nv):
+                hit = np.flatnonzero((lv[:, None] - lij[None, :]) == self.label - lv[a])
+                parts.append(n1 + a * blk + hit)
+            self._packed = np.concatenate(parts).astype(np.int64)
+        return self._packed
+
 
 def excitation_sector(model, no, K):
     """The sector of total momentum ``K`` (an integer 3-vector, in units of the reciprocal lattice of

@@ -114,12 +114,33 @@ class FEAST_EOM_CCSD(EOM_CCSD):
         operators that do not fit one GPU); ``"systems"`` -- the (quadrature node x trial vector)
         linear systems of the contour are dealt out over the ranks, every rank applies the full
         (replicated, never-materialised-V_abcd) operator to its own systems and the only exchanges
-        are the all-reduce of the filtered vectors Q and of H-bar Q (SURVEY 8e, second form)."""
+        are the all-reduce of the filtered vectors Q and of H-bar Q (SURVEY 8e, second form).
+
+        ``sector`` (``model.ueg.excitation_sector``): the states of ONE total momentum of a UEG
+        reference.  The operators are checked and tagged as in ``EOM_CCSD(sector=...)`` (``ValueError``
+        names one that breaks momentum conservation), and every vector the driver holds -- trial
+        vectors, contour sums Q, H-bar Q and every GCROT vector -- is COMPACT: the ``n_sec`` allowed
+        elements of the packed [singles | doubles] layout (``ExcitationSector.packed_index``).  Sigma
+        scatters up to ``max_rhs`` of them into a persistent dense staging stack that carries the
+        sector rules, runs ``SigmaPlan.apply`` on momentum groups and gathers the result (after
+        checking that both outputs still carry the sector rules).  ``max_rhs`` defaults to 16 in a
+        sector: the dense staging (U2, S2 and the Ex temporary of ``apply``, 3 x 16 doubles vectors)
+        then stays under 37 GB at 389 plane waves (v = 362, o = 27).  The seeded start vectors are the
+        reference's dense draws restricted to the sector; ``u_singles`` / ``u_doubles`` come back
+        dense ([v,o] / [v,v,o,o], zero outside the sector, tagged with its rules) and are accepted as
+        start vectors when they lie in the sector (``ValueError`` otherwise).  The K = 0 sector
+        (doubles only) is allowed; an empty sector or one smaller than ``n_trial`` raises
+        ``ValueError``.  ``parallel="systems"`` works in a sector; ``parallel="rows"`` with more than
+        one rank raises ``NotImplementedError``."""
         self.parallel = kwargs.get("parallel", "rows")
         if self.parallel not in ("rows", "systems"):
             raise ValueError("parallel must be 'rows' or 'systems'")
         comm = kwargs.get("comm")
-        super().__init__(no, n_excit=2, comm=comm if self.parallel == "rows" else None)
+        sector = kwargs.get("sector")
+        if sector is not None and self.parallel == "rows" and comm is not None and comm.size > 1:
+            raise NotImplementedError("FEAST-EOM-CCSD in a momentum sector: row-sharded sigma is not available; "
+                                      "use parallel='systems'")
+        super().__init__(no, n_excit=2, comm=comm if self.parallel == "rows" else None, sector=sector)
         self.sys_comm = comm if (self.parallel == "systems" and comm is not None and comm.size > 1) else None
         self.e_c = e_c
         self.e_r = e_r
@@ -133,8 +154,10 @@ class FEAST_EOM_CCSD(EOM_CCSD):
         self.ls_restart = 20         # scipy's default m (inner steps per cycle once the recycle space is full)
         self.ls_recycle = None       # scipy's k: recycled (c, u) pairs kept; None = m, like gcrotmk(k=None)
         self.n_nodes = 8             # feast:97
-        self.max_rhs = 64            # real right-hand sides per batched sigma call
+        # real right-hand sides per batched sigma call (in a sector: per dense staging stack)
+        self.max_rhs = 64 if sector is None else 16
         self.max_systems = None      # systems advanced together (None: all); bounds the Krylov memory
+        self._layout = None          # sector mode: the compact layout and the dense staging stack
         self.u_singles = []
         self.u_doubles = []
         self.eigvals = np.array([self.e_c - self.e_r, self.e_c + self.e_r])
@@ -145,6 +168,63 @@ class FEAST_EOM_CCSD(EOM_CCSD):
     def dump_log(self):
         pass
 
+    # ---- sector layout ----------------------------------------------------
+    def sector_layout(self, nv):
+        """Sector mode: the compact layout of the sector for ``nv`` virtuals, built once -- a dict with
+        ``host`` (``packed_index``, numpy), ``idx`` (the same on the device), ``i1`` / ``i2`` (device
+        offsets of the singles in [v,o] and of the doubles in [v,v,o,o]), ``n1`` (singles in the
+        sector) and ``n`` (all elements).  ``ValueError`` for an empty sector or one smaller than
+        ``n_trial``."""
+        sec = self.sector
+        if self._layout is None or self._layout["nv"] != nv:
+            host = sec.packed_index()
+            if len(host) == 0:
+                raise ValueError("the sector %r holds no excitation" % (sec,))
+            if len(host) < self.n_trial:
+                raise ValueError("n_trial = %d exceeds the %d excitations of the sector %r"
+                                 % (self.n_trial, len(host), sec))
+            n1 = int(np.searchsorted(host, nv * self.no))
+            dev = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.int64)).to(bk.device())
+            self._layout = {"nv": nv, "host": host, "idx": dev(host), "i1": dev(host[:n1]),
+                            "i2": dev(host[n1:] - nv * self.no), "n1": n1, "n": len(host), "staging": None}
+        return self._layout
+
+    def _staging(self, lay, r):
+        """The first ``r`` rows of the dense staging stacks U1 [R,v,o] / U2 [R,v,v,o,o]: zeroed once and
+        tagged with the stacked sector rules (scatters write only allowed elements, so they keep them)."""
+        st = lay["staging"]
+        if st is None or st[0].shape[0] < r:
+            st = lay["staging"] = None                      # free the smaller stack before the larger one
+            sec, nv, no = self.sector, lay["nv"], self.no
+            st = lay["staging"] = [bk.zeros(r, *shape, rule=rule.with_axes([(0, r, 0)] + list(rule.axes)))
+                                   for rule, shape in ((sec.singles_rule(), (nv, no)),
+                                                       (sec.doubles_rule(), (nv, nv, no, no)))]
+        return bk.narrow(st[0], 0, 0, r), bk.narrow(st[1], 0, 0, r)
+
+    def _sigma_compact(self, plan, X):
+        """H-bar on the compact sector vectors X [r, n_sec]: scatter into the staging stack, sigma on
+        momentum groups, gather."""
+        lay = self.sector_layout(plan.nv)
+        n1, r = lay["n1"], X.shape[0]
+        U1, U2 = self._staging(lay, r)
+        if n1:
+            bk.sector_scatter(X[:, :n1], lay["i1"], U1)
+        bk.sector_scatter(X[:, n1:], lay["i2"], U2)
+        k1, k2 = bk.momentum_of(U1), bk.momentum_of(U2)
+        S1, S2 = plan.apply(U1, U2)
+        if k1 is None or k2 is None or bk.momentum_of(S1) != k1 or bk.momentum_of(S2) != k2:
+            raise RuntimeError("sigma in the sector %r lost the sector rule: gathering it would drop weight"
+                               % (self.sector,))
+        Y = bk.empty(r, lay["n"])
+        if n1:
+            bk.sector_gather(S1, lay["i1"], out=Y[:, :n1])
+        bk.sector_gather(S2, lay["i2"], out=Y[:, n1:])
+        return Y
+
+    def _apply_block(self, plan, X):
+        """H-bar on the rows of X: packed dense vectors, or compact ones in a sector."""
+        return plan.apply_packed(X) if self.sector is None else self._sigma_compact(plan, X)
+
     # ---- batched linear solves -------------------------------------------
     def _sigma_c(self, plan, vecs):
         """H-bar applied to a list of _CVec through batched real sigma calls."""
@@ -153,7 +233,7 @@ class FEAST_EOM_CCSD(EOM_CCSD):
             flat += [v.re, v.im]
         out = []
         for lo in range(0, len(flat), self.max_rhs):
-            Y = plan.apply_packed(torch.stack(flat[lo:lo + self.max_rhs]))
+            Y = self._apply_block(plan, torch.stack(flat[lo:lo + self.max_rhs]))
             out += [Y[k] for k in range(Y.shape[0])]
         self.ls_matvecs += len(vecs)
         return [_CVec(out[2 * k], out[2 * k + 1]) for k in range(len(vecs))]
@@ -319,6 +399,8 @@ class FEAST_EOM_CCSD(EOM_CCSD):
     # ---- reference-shaped single solve (used by the parity tests) ---------
     def _gcrotmk(self, l, ze, diag_ai, diag_abij, t_fock_dressed_pq, dict_t_V_dressed, t_T_abij, **kwargs):
         """(Q_singles, Q_doubles) = (ze - H-bar)^-1 u_l as complex numpy arrays, feast:293-350."""
+        if self.sector is not None:
+            raise NotImplementedError("_gcrotmk takes dense vectors; in a sector use solve_shifted_systems")
         plan = self.plan(t_fock_dressed_pq, dict_t_V_dressed, t_T_abij)
         d1, d2 = bk.asdev(diag_ai), bk.asdev(diag_abij)
         diag = torch.cat([d1.reshape(-1), d2.reshape(-1)])
@@ -340,6 +422,22 @@ class FEAST_EOM_CCSD(EOM_CCSD):
             self.sys_comm.all_reduce_sum(t)
         return t
 
+    def _start_vector(self, u_singles, u_doubles):
+        """A user-supplied start vector as one flat device vector (compact in a sector, after checking
+        that it lies in the sector: ``ValueError`` otherwise)."""
+        u1, u2 = bk.asdev(u_singles).contiguous(), bk.asdev(u_doubles).contiguous()
+        sec = self.sector
+        if sec is None:
+            return torch.cat([u1.reshape(-1), u2.reshape(-1)])
+        if not (bk.adopt_momentum(u1, sec.singles_rule()) and bk.adopt_momentum(u2, sec.doubles_rule())):
+            raise ValueError("a start vector has weight outside the sector %r" % (sec,))
+        lay = self.sector_layout(u1.shape[0])
+        out = bk.empty(1, lay["n"])
+        if lay["n1"]:
+            bk.sector_gather(u1.reshape(1, -1), lay["i1"], out=out[:, :lay["n1"]])
+        bk.sector_gather(u2.reshape(1, -1), lay["i2"], out=out[:, lay["n1"]:])
+        return out[0]
+
     def solve(self, t_fock_dressed_pq, dict_t_V_dressed, t_T_abij):
         print_title("FEAST-EOM-CCSD Solver")
         time_init = time.time()
@@ -350,14 +448,18 @@ class FEAST_EOM_CCSD(EOM_CCSD):
         d1 = self.get_diag_singles(t_fock_dressed_pq, dict_t_V_dressed, bk.asdev(t_T_abij))
         d2 = self.get_diag_doubles(t_fock_dressed_pq, dict_t_V_dressed, bk.asdev(t_T_abij))
         diag = torch.cat([d1.reshape(-1), d2.reshape(-1)])
+        sec = self.sector
+        if sec is not None:                                 # every vector below is compact
+            lay = self.sector_layout(nv)
+            diag = bk.sector_gather(diag[None], lay["idx"])[0]
 
         print_logging_info("Initialising u tensors...", level=1)
-        U = [torch.cat([bk.asdev(a).reshape(-1), bk.asdev(b).reshape(-1)])
-             for a, b in zip(self.u_singles, self.u_doubles)]
+        U = [self._start_vector(a, b) for a, b in zip(self.u_singles, self.u_doubles)]
         for _ in range(self.n_excit):                       # same RNG call order as feast:89-91
             a = 0.5 - np.random.rand(nv, no)
             b = (0.5 - np.random.rand(nv, nv, no, no)) * 0.01
-            U.append(bk.asdev(np.concatenate([a.ravel(), b.ravel()])))
+            u = np.concatenate([a.ravel(), b.ravel()])
+            U.append(bk.asdev(u if sec is None else u[lay["host"]]))
         if self.sys_comm is not None:                       # one start for all ranks: rank 0's
             for u in U:
                 if self.sys_comm.rank != 0:
@@ -403,7 +505,7 @@ class FEAST_EOM_CCSD(EOM_CCSD):
             cols = self._share(m)
             for lo in range(0, len(cols), self.max_rhs):
                 sel = cols[lo:lo + self.max_rhs]
-                Wq[sel] = plan.apply_packed(Qs[sel])
+                Wq[sel] = self._apply_block(plan, Qs[sel])
             self._sum_over_ranks(Wq)
             H_proj, B = np.zeros((m, m)), np.zeros((m, m))
             hb = [(bk.dots(Q, Wq[i]), bk.dots(Q, Q[i])) for i in range(m)]
@@ -431,8 +533,15 @@ class FEAST_EOM_CCSD(EOM_CCSD):
                                level=1)
             e_norm_prev = e_norm
         self.iterations = it + 1
-        self.u_singles = [u[:n1].view(nv, no) for u in U]
-        self.u_doubles = [u[n1:].view(nv, nv, no, no) for u in U]
+        if sec is None:
+            self.u_singles = [u[:n1].view(nv, no) for u in U]
+            self.u_doubles = [u[n1:].view(nv, nv, no, no) for u in U]
+        else:                                               # dense, zero outside the sector, tagged
+            ns = lay["n1"]
+            self.u_singles = [bk.sector_scatter(u[:ns], lay["i1"], bk.zeros(nv, no, rule=sec.singles_rule()))
+                              for u in U]
+            self.u_doubles = [bk.sector_scatter(u[ns:], lay["i2"],
+                                                bk.zeros(nv, nv, no, no, rule=sec.doubles_rule())) for u in U]
         print_logging_info(f"FEAST-EOM-CCSD finished in {time.time() - time_init:.2f} seconds.", level=0)
         self.e_excit = self.eigvals
         return self.eigvals

@@ -27,6 +27,8 @@ from .feast_eom_ccsd import FEAST_EOM_CCSD, _CVec, get_gauss_legendre_quadrature
 
 class RT_EOM_CCSD(FEAST_EOM_CCSD):
     def __init__(self, no, e_c=0., e_r=1, dt=0.1, tol=1e-12, max_iter=100, **kwargs):
+        if kwargs.get("sector") is not None:
+            raise NotImplementedError("RT-EOM-CCSD in a momentum sector is not available")
         super().__init__(no, e_c=e_c, e_r=e_r, n_trial=1, max_iter=max_iter, tol=tol, **kwargs)
         self.dt = dt
         self.u_singles = None
