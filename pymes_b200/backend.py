@@ -554,8 +554,9 @@ def blocked_enabled():
 def blocked_companion(t):
     """The never-materialised twin of a STORED integral block (``UEG.eval_2b_blocks`` attaches one
     to V_iabc / V_aibc: their compressed values are 1/v of the block), for the contractions that
-    can run momentum-blocked; None when there is none or the blocked path is switched off."""
-    return getattr(t, "_pmb_blocked", None) if _BLOCKED[0] else None
+    can run momentum-blocked; None when there is none, the blocked path is switched off, or the
+    block was edited in place since (its twin holds the old values)."""
+    return getattr(t, "_pmb_blocked", None) if _BLOCKED[0] and block_rule(t) is not None else None
 
 
 def _column_groups(n_sub, ext, bstr, cstr):
@@ -650,8 +651,10 @@ class Momentum:
         return lab - self.total if d == 0 and self.total else lab
 
 
-def _set_momentum(t, key):
-    t._pmb_mom = (key, t._version) if key is not None else None
+def _set_momentum(t, key, block=False):
+    """Tag ``t`` with the rule ``key`` (None: untagged); ``block`` marks a stored integral block
+    (:func:`tag_block`).  One version stamp serves both: an in-place edit ends the two."""
+    t._pmb_mom = (key, t._version, block) if key is not None else None
 
 
 def momentum_of(x):
@@ -684,9 +687,11 @@ def adopt_momentum(t, key, host=None):
     """Tag ``t`` (a tensor that enters from outside) with the rule ``key`` if and only if every
     element the rule forbids is exactly zero (``pmb_momentum_residue``: one pass over the tensor).
     ``host``: the same values as a numpy array the caller holds anyway (e.g. the Fock matrix); they
-    are checked there instead.  Returns True when it was tagged."""
+    are checked there instead.  Returns True when it was tagged.  A stored integral block adopted
+    under its own rule stays one (:func:`block_rule`)."""
     if key is None or not isinstance(t, torch.Tensor) or t.dim() != len(key.axes) or not 1 <= t.dim() <= 4:
         return False
+    block = block_rule(t) == key
     if any(int(n) != a[1] for n, a in zip(t.shape, key.axes)):
         raise ValueError("momentum rule %s does not fit a tensor of shape %s" % (key.axes, tuple(t.shape)))
     if host is not None:
@@ -697,11 +702,11 @@ def adopt_momentum(t, key, host=None):
         for d in range(t.dim()):
             total = np.add.outer(total, key.labels(d))
         ok = not np.any(host[total != 0] != 0)           # NaN != 0: not adopted
-        _set_momentum(t, key if ok else None)
+        _set_momentum(t, key if ok else None, ok and block)
         return ok
     if t.numel() == 0:
         # no element can break the rule (and pmb_momentum_residue takes no extent of 0)
-        _set_momentum(t, key)
+        _set_momentum(t, key, block)
         return True
     labels = torch.from_numpy(np.concatenate([key.labels(d) for d in range(t.dim())])).to(device())
     res = zeros(1)
@@ -709,7 +714,7 @@ def adopt_momentum(t, key, host=None):
                                                  _lib.I64x4(*_pad4r(t.stride(), 0)), _ptr(t), _ptr(labels),
                                                  _ptr(res), _stream()), "pmb_momentum_residue")
     ok = float(res.item()) == 0.0
-    _set_momentum(t, key if ok else None)
+    _set_momentum(t, key if ok else None, ok and block)
     return ok
 
 
@@ -801,18 +806,21 @@ def _derive(out_sub, terms, old, accumulate):
     return min(cands, key=lambda k: k.axes)
 
 
-def tag_geom(t, geom):
-    """Attach the (p,q,r,s) geometry of a stored integral block to its tensor (see
-    ``model.ueg.MomentumGeom``) together with its momentum rule; returns the tensor."""
-    t._pmb_geom = (geom, t._version)
-    _set_momentum(t, geom.momentum())
+def tag_block(t, rule):
+    """Mark ``t`` as a stored integral block whose elements obey ``rule`` (``UEG.eval_2b_blocks``):
+    products of such a block with an untagged operand run on its momentum groups
+    (``pmb_blocked_contract``, ``pmb_gather_expand``).  Returns the tensor."""
+    _set_momentum(t, rule, block=True)
     return t
 
 
-def geom_of(t):
-    """The live geometry tag of a stored integral block (None after an in-place edit)."""
-    tag = getattr(t, "_pmb_geom", None) if isinstance(t, torch.Tensor) else None
-    if tag is None or tag[1] != t._version:
+def block_rule(t):
+    """The live rule of a stored integral block (:func:`tag_block`); None for any other tensor and
+    after an in-place edit.  :func:`narrow` and :func:`copy` keep the mark, every backend write and
+    :func:`permute` end it: amplitudes, intermediates and permuted views take the paths their rules
+    alone select."""
+    tag = getattr(t, "_pmb_mom", None) if isinstance(t, torch.Tensor) else None
+    if tag is None or tag[1] != t._version or not tag[2]:
         return None
     return tag[0]
 
@@ -820,12 +828,9 @@ def geom_of(t):
 def narrow(t, dim, lo, n):
     """``t.narrow(dim, lo, n)`` that keeps the tags of ``t``, restricted to the view."""
     out = t.narrow(dim, lo, n)
-    g = geom_of(t)
-    if g is not None:
-        out._pmb_geom = (g.narrow(dim, lo, n), out._version)
     k = momentum_of(t)
     if k is not None:
-        _set_momentum(out, k.narrow(dim, lo, n))
+        _set_momentum(out, k.narrow(dim, lo, n), block_rule(t) is not None)
     out._pmb_parent = (t, int(dim), int(lo), int(n))
     return out
 
@@ -843,13 +848,13 @@ def _structured(x):
     """Does ``x`` carry a block-diagonal momentum structure ``pmb_blocked_contract`` can use?"""
     if isinstance(x, GeneratedOperand):
         return x.blocked_lists() is not None
-    return geom_of(x) is not None
+    return block_rule(x) is not None
 
 
 def _blocked_term(out_sub, term):
     """``(alpha, sa, S, sb, D, m_axes, k_axes)`` if this term can go to ``pmb_blocked_contract``:
     S a momentum-structured 4-index operand (a generated block with block lists, or a stored
-    block with a geometry tag) with two of its indices in the output (``m_axes``, rows) and two
+    integral block, :func:`block_rule`) with two of its indices in the output (``m_axes``, rows) and two
     contracted with D (``k_axes``, entries); every other index of D an output index.  A generated
     operand only in its native split (p,q | r,s).  Else None."""
     if not _BLOCKED[0]:
@@ -898,7 +903,7 @@ def _run_blocked(out_sub, term, out, beta):
         L = A.blocked_lists()
         values, a_moff, a_koff = L["values"], L["a_moff"], L["a_koff"]
     else:
-        L = geom_of(A).lists(m_axes, k_axes)
+        L = block_lists(block_rule(A), m_axes, k_axes)
         astr = A.stride()
         akey = ("a", astr[m_axes[0]], astr[m_axes[1]], astr[k_axes[0]], astr[k_axes[1]])
         aoffs = L["offsets"].get(akey)
@@ -948,6 +953,44 @@ def set_gather(flag):
     return old
 
 
+def partner_tables(S, y_axis):
+    """For a contiguous stored integral block ``S`` and one of its axes ``y_axis``: ``idx[x0,x1,x2]``
+    = the local index along that axis of the ONE orbital whose label completes the other three to
+    the block's rule (:func:`block_rule`), or -1, and ``val[x0,x1,x2] = S[x0,x1,x2 | idx]`` (0 where
+    there is none) -- what ``pmb_gather_expand`` reads instead of the block.  (x0,x1,x2) are the
+    other three axes in S's own order.  Device tensors, cached on the tensor that owns S's storage
+    (they go with the block, and a row block narrowed again every sweep finds them) until the
+    storage is next written."""
+    rule = block_rule(S)
+    if rule is None or not S.is_contiguous():
+        raise ValueError("partner tables need a contiguous stored integral block")
+    owner = S if S._base is None else S._base
+    cache = getattr(owner, "_pmb_partner", None)
+    if cache is None or cache[0] != S._version:
+        cache = owner._pmb_partner = (S._version, {})
+    key = (rule, int(y_axis), S.data_ptr())
+    tab = cache[1].get(key)
+    if tab is None:
+        others = [ax for ax in range(4) if ax != y_axis]
+        l0, l1, l2 = (rule.labels(ax) for ax in others)
+        want = -(l0[:, None, None] + l1[None, :, None] + l2[None, None, :]).reshape(-1)
+        ly = rule.labels(y_axis)
+        order = np.argsort(ly)
+        pos = np.minimum(np.searchsorted(ly[order], want), len(ly) - 1)
+        hit = ly[order][pos] == want
+        idx = np.where(hit, order[pos], -1).astype(np.int32)
+        # flat position in S of (x0,x1,x2 | idx)
+        grid = np.meshgrid(*[np.arange(S.shape[ax], dtype=np.int64) for ax in others], indexing="ij")
+        flat = sum(g * S.stride(ax) for g, ax in zip(grid, others)).reshape(-1)
+        flat = flat + np.maximum(idx, 0).astype(np.int64) * S.stride(y_axis)
+        idx_d = torch.from_numpy(idx).to(device())
+        val = torch.index_select(S.reshape(-1), 0, torch.from_numpy(flat).to(device()))
+        val = torch.where(idx_d >= 0, val, torch.zeros_like(val))
+        tab = cache[1][key] = dict(idx=idx_d, val=val, ext=tuple(int(S.shape[ax]) for ax in others),
+                                   n_hit=int(hit.sum()))
+    return tab
+
+
 def _try_gather(out_sub, terms, out, beta):
     """``out[x0,x1,x2,j] = beta*out + alpha * sum_y S[x0,x1,x2|y] D[y,j]`` for a stored, tagged UEG
     integral block S (three of its indices in the output, one summed) and a two-index D (T1): one
@@ -956,15 +999,14 @@ def _try_gather(out_sub, terms, out, beta):
     if not (_BLOCKED[0] and _GATHER[0]) or len(terms) != 1 or len(out_sub) != 4 or len(set(out_sub)) != 4:
         return None
     alpha, sa, A, sb, B = terms[0]
-    if geom_of(A) is None:
+    if block_rule(A) is None:
         sa, A, sb, B = sb, B, sa, A
-    g = geom_of(A)
-    if g is None or isinstance(B, (GeneratedOperand, LinearOperator)) or len(sa) != 4 or len(sb) != 2:
+    if block_rule(A) is None or isinstance(B, (GeneratedOperand, LinearOperator)) or len(sa) != 4 or len(sb) != 2:
         return None
     if len(set(sa)) != 4 or len(set(sb)) != 2 or not A.is_contiguous():
         return None
     B = asdev(B)
-    if B.dim() != 2 or geom_of(B) is not None:
+    if B.dim() != 2 or block_rule(B) is not None:
         return None
     ys = [ch for ch in sa if ch in sb]
     if len(ys) != 1 or ys[0] in out_sub:
@@ -990,7 +1032,7 @@ def _try_gather(out_sub, terms, out, beta):
     elif out.device != device():
         raise RuntimeError("pymes_b200: output tensor lives on %s, the kernels write to %s "
                            "(there is no CPU fallback)" % (out.device, device()))
-    tab = g.partner_tables(A, sa.index(y))
+    tab = partner_tables(A, sa.index(y))
     d = _lib.Gather()
     d.val, d.idx, d.D, d.out = tab["val"].data_ptr(), tab["idx"].data_ptr(), B.data_ptr(), out.data_ptr()
     xe = tab["ext"]
@@ -1067,6 +1109,58 @@ def _side_members(k, axes, sign, shift, common):
     pos = pos[np.argsort(lab[pos], kind="stable")]
     _keys, first, cnt = np.unique(lab[pos], return_index=True, return_counts=True)
     return pos, first, cnt
+
+
+def block_groups(rule, m_axes, k_axes):
+    """The 4-index tensor with momentum rule ``rule`` as the matrix [rows = axes ``m_axes``, entries =
+    axes ``k_axes``] is block diagonal: a row and an entry can meet only where their labels cancel.
+    Returns ``(row_pos, ent_pos, g_row0, g_rows, g_ent0, g_ents)``: the flat positions (C order over
+    the side's axes) of the rows / entries of the groups present on both sides, sorted by group
+    (index order inside a group), and each group's first position and length in the two lists."""
+    sides = ((rule, m_axes, 1, -rule.total), (rule, k_axes, -1, 0))
+    common = np.intersect1d(_side_keys(*sides[0]), _side_keys(*sides[1]))
+    (r_pos, r_first, r_cnt), (e_pos, e_first, e_cnt) = (_side_members(*s_, common) for s_ in sides)
+    return r_pos, e_pos, r_first, r_cnt, e_first, e_cnt
+
+
+def blocked_tiles(g_first, g_cnt, g_e0, g_en, tile_rows=64):
+    """Row tiles of ``pmb_blocked_contract``: every group's rows in equal pieces of whole 8-row
+    fragments, at most ``tile_rows`` each; {first row, rows, first entry, entries} per tile,
+    long groups first."""
+    pieces = -(-g_cnt // tile_rows)
+    size = -(-g_cnt // np.maximum(pieces, 1))
+    size = np.minimum(-(-size // 8) * 8, tile_rows)
+    pieces = -(-g_cnt // np.maximum(size, 1))
+    grp = np.repeat(np.arange(len(g_cnt)), pieces)
+    within = np.arange(len(grp)) - np.repeat(np.cumsum(pieces) - pieces, pieces)
+    t_m0 = g_first[grp] + within * size[grp]
+    t_mn = np.minimum(size[grp], g_cnt[grp] - within * size[grp])
+    tiles = np.stack([t_m0, t_mn, g_e0[grp], g_en[grp]], axis=1).astype(np.int32)
+    return np.ascontiguousarray(tiles[np.argsort(-tiles[:, 3], kind="stable")])
+
+
+_LIST_CACHE = {}
+
+
+def block_lists(rule, m_axes=(0, 1), k_axes=(2, 3)):
+    """Lists of ``pmb_blocked_contract`` for a 4-index tensor with momentum rule ``rule`` split as
+    :func:`block_groups`: the index pairs of the rows / entries (numpy int64, sorted by group), the
+    device tile table and a cache for the offset tables derived from them.  Cached by value (a
+    sharded sweep narrows the same blocks every iteration)."""
+    key = (rule, tuple(m_axes), tuple(k_axes), str(device()))
+    L = _LIST_CACHE.get(key)
+    if L is None:
+        r_pos, e_pos, g_first, g_cnt, g_e0, g_en = block_groups(rule, m_axes, k_axes)
+        ext = [n for _lo, n, _sg in rule.axes]
+        tiles = blocked_tiles(g_first, g_cnt, g_e0, g_en)
+        L = _LIST_CACHE[key] = dict(
+            row_i0=r_pos // ext[m_axes[1]], row_i1=r_pos % ext[m_axes[1]],
+            ent_j0=e_pos // ext[k_axes[1]], ent_j1=e_pos % ext[k_axes[1]],
+            tiles=torch.from_numpy(tiles).to(device()), n_tiles=len(tiles),
+            nnz=int((g_cnt * g_en).sum()), n_groups=len(g_cnt), offsets={},
+            # every row meets at least one entry: a fresh output needs no clearing
+            rows_covered=int(g_cnt.sum()) == ext[m_axes[0]] * ext[m_axes[1]])
+    return L
 
 
 def _side_offsets(pos, ext, *strides):
@@ -1396,9 +1490,9 @@ def axpby(alpha, src, beta=0.0, out=None):
 def copy(src):
     """A copy keeps the tags of its source (a copy of a stored integral block IS the block)."""
     out = axpby(1.0, src)
-    g = geom_of(src)
-    if g is not None:
-        out._pmb_geom = (g, out._version)
+    rule = block_rule(src)
+    if rule is not None:
+        tag_block(out, rule)
     return out
 
 

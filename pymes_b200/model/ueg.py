@@ -383,8 +383,8 @@ class UEG:
             if key in virtual:
                 out[key] = self.virtual_block(lo, ext, W0a=W0a, W1a=W1a, W0s=W0s)
             else:
-                out[key] = bk.tag_geom(self.build_block(lo, ext, W0a=W0a, W1a=W1a, W0s=W0s, out=pre.get(key)),
-                                       MomentumGeom(self, lo, ext))
+                out[key] = bk.tag_block(self.build_block(lo, ext, W0a=W0a, W1a=W1a, W0s=W0s, out=pre.get(key)),
+                                        momentum_rule(self, lo, ext))
                 if key in BLOCKED_COMPANIONS:
                     # stored AND available as compressed values (1/v of the block): V.tau of the
                     # T1 dressing runs momentum-blocked (solver.ccsd.pair_with_tau)
@@ -526,51 +526,29 @@ def momentum_groups(k_int, imax, lo, ext, m_axes=(0, 1), k_axes=(2, 3)):
     elements and the few aliased ones the reference produces as well (a component beyond imax
     carries into the next digit).  With signs (+,+,-,-) for (p,q,r,s), a row and an entry can
     meet where  sum_rows sign.l = - sum_entries sign.l ; rows and entries with the same key form a
-    group.  Returns ``(row_ord, ent_ord, g_row0, g_rows, g_ent0, g_ents)``: the permutations
-    that sort the rows i0*ext[m1]+i1 / the entries j0*ext[k1]+j1 by group (stable: index order
-    inside a group) and, per group present on BOTH sides, its first position and length in the two
-    sorted lists.  ``(g_rows * g_ents).sum()`` is the number of candidate non-zeros (54e / 515
-    plane waves, V_abcd: 3.3e7 of 5.7e10)."""
+    group.  Returns ``(row_ord, ent_ord, g_row0, g_rows, g_ent0, g_ents)``: the rows i0*ext[m1]+i1 /
+    the entries j0*ext[k1]+j1 of the groups present on BOTH sides, sorted by group (index order
+    inside a group), and per group its first position and length in the two lists
+    (``backend.block_groups``).  ``(g_rows * g_ents).sum()`` is the number of candidate non-zeros
+    (54e / 515 plane waves, V_abcd: 3.3e7 of 5.7e10)."""
     if sorted(tuple(m_axes) + tuple(k_axes)) != [0, 1, 2, 3]:
         raise ValueError("row and entry axes must split (p,q,r,s)")
-    k = np.asarray(k_int).astype(np.int64)
+    return bk.block_groups(bk.Momentum(linearise(k_int, imax), zip(lo, ext, SIGNS)), m_axes, k_axes)
+
+
+def linearise(k, imax):
+    """l(k) = n^2 x + n y + z (n = 2 imax + 1) of integer momenta ``k[..., 3]``: the label the
+    reference's index lookup conserves (see :func:`momentum_groups`)."""
+    k = np.asarray(k).astype(np.int64)
     n = 2 * int(imax) + 1
-    lin = n * n * k[:, 0] + n * k[:, 1] + k[:, 2]
-    l = [SIGNS[ax] * lin[lo[ax]:lo[ax] + ext[ax]] for ax in range(4)]
-    row_key = (l[m_axes[0]][:, None] + l[m_axes[1]][None, :]).reshape(-1)
-    ent_key = -(l[k_axes[0]][:, None] + l[k_axes[1]][None, :]).reshape(-1)
-    row_ord = np.argsort(row_key, kind="stable")
-    ent_ord = np.argsort(ent_key, kind="stable")
-    rk, r_first, r_cnt = np.unique(row_key[row_ord], return_index=True, return_counts=True)
-    ek, e_first, e_cnt = np.unique(ent_key[ent_ord], return_index=True, return_counts=True)
-    _common, ri, ei = np.intersect1d(rk, ek, assume_unique=True, return_indices=True)
-    return row_ord, ent_ord, r_first[ri], r_cnt[ri], e_first[ei], e_cnt[ei]
-
-
-def blocked_tiles(g_first, g_cnt, g_e0, g_en, tile_rows=64):
-    """Row tiles of ``pmb_blocked_contract``: every group's rows in equal pieces of whole 8-row
-    fragments, at most ``tile_rows`` each; {first row, rows, first entry, entries} per tile,
-    long groups first."""
-    pieces = -(-g_cnt // tile_rows)
-    size = -(-g_cnt // np.maximum(pieces, 1))
-    size = np.minimum(-(-size // 8) * 8, tile_rows)
-    pieces = -(-g_cnt // np.maximum(size, 1))
-    grp = np.repeat(np.arange(len(g_cnt)), pieces)
-    within = np.arange(len(grp)) - np.repeat(np.cumsum(pieces) - pieces, pieces)
-    t_m0 = g_first[grp] + within * size[grp]
-    t_mn = np.minimum(size[grp], g_cnt[grp] - within * size[grp])
-    tiles = np.stack([t_m0, t_mn, g_e0[grp], g_en[grp]], axis=1).astype(np.int32)
-    return np.ascontiguousarray(tiles[np.argsort(-tiles[:, 3], kind="stable")])
+    return n * n * k[..., 0] + n * k[..., 1] + k[..., 2]
 
 
 def linear_momenta(model):
-    """l(k) = n^2 x + n y + z (n = 2 imax + 1) of every orbital, the label the reference's index
-    lookup conserves (see :func:`momentum_groups`); cached on the model."""
+    """:func:`linearise` of every orbital's momentum; cached on the model."""
     lin = model.__dict__.get("_pmb_lin")
     if lin is None:
-        k = model.k_int().astype(np.int64)
-        n = 2 * int(model.imax) + 1
-        lin = model.__dict__["_pmb_lin"] = n * n * k[:, 0] + n * k[:, 1] + k[:, 2]
+        lin = model.__dict__["_pmb_lin"] = linearise(model.k_int(), model.imax)
     return lin
 
 
@@ -652,9 +630,7 @@ def excitation_sector(model, no, K):
     K = np.asarray(K)
     if K.shape != (3,) or not np.issubdtype(K.dtype, np.integer):
         raise ValueError("K must be an integer 3-vector")
-    n = 2 * int(model.imax) + 1
-    label = n * n * int(K[0]) + n * int(K[1]) + int(K[2])
-    return ExcitationSector(linear_momenta(model), no, label, K)
+    return ExcitationSector(linear_momenta(model), no, int(linearise(K, model.imax)), K)
 
 
 def excitation_sectors(model, no):
@@ -690,88 +666,6 @@ def momentum_rule(model, lo, ext, signs=SIGNS):
     return bk.Momentum(linear_momenta(model), zip(lo, ext, signs))
 
 
-class MomentumGeom:
-    """Where a STORED integral block sits in (p,q,r,s) orbital space: attached to the tensors
-    ``UEG.eval_2b_blocks`` returns (``backend.tag_geom``) so that contractions whose structured
-    operand is such a block can run on its diagonal momentum blocks (``pmb_blocked_contract``).
-    The structure is a property of the integral generator; the amplitudes' structure is derived
-    from it (``backend.Momentum``) or verified, never assumed."""
-
-    def __init__(self, model, lo, ext):
-        self.model, self.lo, self.ext = model, tuple(int(x) for x in lo), tuple(int(x) for x in ext)
-        self._lists, self._narrowed = {}, {}
-
-    def narrow(self, dim, lo, n):
-        """Geometry of ``block.narrow(dim, lo, n)`` (cached: a sharded sweep narrows the same blocks
-        every iteration, and the lists / device tables hang off the geometry object)."""
-        key = (int(dim), int(lo), int(n))
-        sub = self._narrowed.get(key)
-        if sub is None:
-            new_lo, new_ext = list(self.lo), list(self.ext)
-            new_lo[dim] += int(lo)
-            new_ext[dim] = int(n)
-            sub = self._narrowed[key] = MomentumGeom(self.model, new_lo, new_ext)
-        return sub
-
-    def momentum(self):
-        return momentum_rule(self.model, self.lo, self.ext)
-
-    def partner_tables(self, S, y_axis):
-        """For the stored block ``S`` (contiguous, this geometry) and one summed axis ``y_axis``:
-        ``idx[x0,x1,x2]`` = the local index along that axis of the ONE orbital the reference's lookup
-        can pair with the other three indices (``l_y = -sign_y * sum_others sign.l``, see
-        :func:`momentum_groups`), or -1, and ``val[x0,x1,x2] = S[x0,x1,x2 | idx]`` (0 where there is
-        none) -- what ``pmb_gather_expand`` reads instead of the block.  (x0,x1,x2) are the other
-        three axes in S's own order.  Device tensors, cached per (block memory, axis)."""
-        key = ("partner", int(S.data_ptr()), int(y_axis))
-        tab = self._lists.get(key)
-        if tab is None:
-            k = self.model.k_int().astype(np.int64)
-            n = 2 * int(self.model.imax) + 1
-            lin = n * n * k[:, 0] + n * k[:, 1] + k[:, 2]
-            lo, ext = self.lo, self.ext
-            others = [ax for ax in range(4) if ax != y_axis]
-            l = [SIGNS[ax] * lin[lo[ax]:lo[ax] + ext[ax]] for ax in others]
-            want = -SIGNS[y_axis] * (l[0][:, None, None] + l[1][None, :, None] + l[2][None, None, :])
-            ly = lin[lo[y_axis]:lo[y_axis] + ext[y_axis]]
-            order = np.argsort(ly)
-            pos = np.searchsorted(ly[order], want.reshape(-1))
-            pos = np.minimum(pos, len(ly) - 1)
-            hit = ly[order][pos] == want.reshape(-1)
-            idx = np.where(hit, order[pos], -1).astype(np.int32)
-            # flat position in S (C order of its own shape) of (x0,x1,x2 | idx)
-            stride = [int(np.prod(ext[ax + 1:])) for ax in range(4)]
-            grid = np.meshgrid(*[np.arange(ext[ax], dtype=np.int64) for ax in others], indexing="ij")
-            flat = sum(g * stride[ax] for g, ax in zip(grid, others)).reshape(-1)
-            flat = flat + np.maximum(idx, 0).astype(np.int64) * stride[y_axis]
-            dev = bk.device()
-            idx_d = torch.from_numpy(idx).to(dev)
-            val = torch.index_select(S.reshape(-1), 0, torch.from_numpy(flat).to(dev))
-            val = torch.where(idx_d >= 0, val, torch.zeros_like(val))
-            tab = self._lists[key] = dict(idx=idx_d, val=val, ext=tuple(ext[ax] for ax in others),
-                                          others=tuple(others), n_hit=int(hit.sum()), keep=S)
-        return tab
-
-    def lists(self, m_axes=(0, 1), k_axes=(2, 3)):
-        """Host lists (numpy int64 index pairs of the rows / entries, sorted by group), the device
-        tile table and a cache for the offset tables derived from them."""
-        key = (tuple(m_axes), tuple(k_axes))
-        L = self._lists.get(key)
-        if L is None:
-            ext = self.ext
-            row_ord, ent_ord, g_first, g_cnt, g_e0, g_en = momentum_groups(
-                self.model.k_int(), self.model.imax, self.lo, ext, m_axes, k_axes)
-            tiles = blocked_tiles(g_first, g_cnt, g_e0, g_en)
-            L = dict(row_i0=(row_ord // ext[m_axes[1]]).astype(np.int64), row_i1=(row_ord % ext[m_axes[1]]).astype(np.int64),
-                     ent_j0=(ent_ord // ext[k_axes[1]]).astype(np.int64), ent_j1=(ent_ord % ext[k_axes[1]]).astype(np.int64),
-                     tiles=torch.from_numpy(tiles).to(bk.device()), n_tiles=len(tiles),
-                     nnz=int((g_cnt * g_en).sum()), n_groups=len(g_cnt), offsets={},
-                     # every row meets at least one entry: a fresh output needs no clearing
-                     rows_covered=int(g_cnt.sum()) == ext[m_axes[0]] * ext[m_axes[1]])
-            self._lists[key] = L
-        return L
-
-
 # stored blocks that also get a never-materialised twin (``backend.blocked_companion``)
 BLOCKED_COMPANIONS = ("iabc", "aibc")
 
@@ -800,10 +694,7 @@ class VirtualBlock(bk.GeneratedOperand):
         self.nz = model.build_nz(self.lo, self.shape, *self.tables) if self.compressed else None
         st = model._device_state()
         if "lin" not in st:
-            n = 2 * model.imax + 1
-            k = model.k_int().astype(np.int64)
-            lin = (n * n * k[:, 0] + n * k[:, 1] + k[:, 2]).astype(np.int32)
-            st["lin"] = torch.from_numpy(lin).to(bk.device())
+            st["lin"] = torch.from_numpy(linearise(model.k_int(), model.imax).astype(np.int32)).to(bk.device())
         self.lin = st["lin"]
 
     def rows(self, dim, lo, n):
@@ -825,15 +716,14 @@ class VirtualBlock(bk.GeneratedOperand):
     def blocked_lists(self):
         """The block as the matrix [(p,q),(r,s)] is block diagonal in the (linearised) total
         momentum, see :func:`momentum_groups` (ueg.py:395-404).  Returns the lists of
-        :meth:`MomentumGeom.lists` plus the operand side of ``pmb_blocked_contract``: the compressed
+        ``backend.block_lists`` plus the operand side of ``pmb_blocked_contract``: the compressed
         values ``nz[p,q,r]`` and the row / entry offsets into them (the s index is implied by the
         group).  Needs the compressed values; None otherwise."""
         if self.nz is None:
             return None
         L = self.__dict__.get("_blocked")
         if L is None:
-            geom = self.__dict__.setdefault("_geom", MomentumGeom(self.model, self.lo, self.shape))
-            L = dict(geom.lists((0, 1), (2, 3)))
+            L = dict(bk.block_lists(self.momentum()))
             ext, dev = self.shape, bk.device()
             L["values"] = self.nz
             L["a_moff"] = torch.from_numpy((L["row_i0"] * ext[1] + L["row_i1"]) * ext[2]).to(dev)

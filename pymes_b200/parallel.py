@@ -121,7 +121,7 @@ class Shard:
                              % (nv, comm.size))
 
     def rows(self, t, dim=0):
-        return bk.narrow(t, dim, self.lo, self.na)       # keeps the geometry tag of a stored V block
+        return bk.narrow(t, dim, self.lo, self.na)       # keeps the block mark of a stored V block
 
     def gather(self, local):
         return self.comm.all_gather_rows(local, self.nv, self.max_rows)

@@ -585,7 +585,7 @@ def test_momentum_blocked_contractions(n_ele, cutoff):
 
 @pytest.mark.parametrize("n_ele,cutoff", [(14, 5.0), (54, 7.0), (54, 10.0)])
 def test_momentum_blocked_stored_blocks(n_ele, cutoff):
-    """Stored integral blocks with a geometry tag: every 2 + 2 split of the ring-type products of the
+    """Stored integral blocks with the block mark: every 2 + 2 split of the ring-type products of the
     doubles residual (ccd.py:180,189,202,233,234,238) runs on the diagonal momentum blocks and equals
     the dense kernel and a cuBLAS product of the same operands; narrowed row blocks (sharded runs);
     fresh outputs whose rows are not all covered."""

@@ -1149,8 +1149,8 @@ def test_momentum_groups_follow_the_reference_index_lookup():
         assert int((g_rn * g_en).sum()) == int(hit.sum())      # and nothing else is visited
 
 
-def test_momentum_blocked_stored_blocks_host_logic(cpu_abi):
-    """Stored integral blocks carry a geometry tag (``UEG.eval_2b_blocks``): contractions that split
+def test_block_marked_stored_blocks_host_logic(cpu_abi):
+    """Stored integral blocks carry a block mark (``UEG.eval_2b_blocks``): contractions that split
     their four indices 2 + 2 between output and sum run on the diagonal momentum blocks for ANY
     such split (the ring-type products of ccd.py:189-204,233-240 with V_ijab / V_iajb), including
     narrowed row blocks; patterns the blocked kernel cannot take stay on the dense kernel."""
@@ -1164,7 +1164,7 @@ def test_momentum_blocked_stored_blocks_host_logic(cpu_abi):
     nv = nP - no
     parts = [("only_non_hermi_2b", m.trunc), ("effect_2b", m.trunc)]
     dV = m.eval_2b_blocks(no, ["ijab", "iajb", "iabj", "klij", "abic"], parts)
-    assert all(bk.geom_of(v) is not None for v in dV.values())
+    assert all(bk.block_rule(v) is not None for v in dV.values())
     rng = np.random.default_rng(9)
     T = _t(rng.standard_normal((nv, nv, no, no)))
     calls = {"blocked": 0, "dense": 0}
@@ -1197,7 +1197,7 @@ def test_momentum_blocked_stored_blocks_host_logic(cpu_abi):
         bk.set_gather(old_gather)
     # row blocks keep their tag through backend.narrow (parallel.Shard.rows)
     part = bk.narrow(V_ijab, 2, 2, 3)
-    assert bk.geom_of(part).lo[2] == no + 2 and bk.geom_of(part).ext[2] == 3
+    assert bk.block_rule(part).axes[2] == (no + 2, 3, -1)
     b0 = calls["blocked"]
     got = bk.contract("klcd,dblj->cbkj", part, T)
     np.testing.assert_allclose(_n(got), np.einsum("klcd,dblj->cbkj", _n(V_ijab)[:, :, 2:5], _n(T)), rtol=0, atol=1e-12)
@@ -1205,8 +1205,8 @@ def test_momentum_blocked_stored_blocks_host_logic(cpu_abi):
     # the undressed V_ijab "dressed" is a tagged copy; dressed blocks with T1 terms are not tagged
     T1 = _t(rng.standard_normal((nv, no)))
     full = m.eval_2b_blocks(no, ["ijab", "ijka", "ijak", "iajb", "iacb"] if False else ["ijab", "ijka"], parts)
-    assert bk.geom_of(ccsd.dressed_block("ijab", T1, full)) is not None
-    assert bk.geom_of(ccsd.dressed_block("ijka", T1, full)) is None
+    assert bk.block_rule(ccsd.dressed_block("ijab", T1, full)) is not None
+    assert bk.block_rule(ccsd.dressed_block("ijka", T1, full)) is None
     # accumulate into an existing tensor with a coefficient, multi-term call with a dense term
     R0 = rng.standard_normal((nv, nv, no, no))
     R = _t(R0.copy())
@@ -1216,7 +1216,7 @@ def test_momentum_blocked_stored_blocks_host_logic(cpu_abi):
     np.testing.assert_allclose(_n(R), want, rtol=0, atol=1e-12)
 
 
-def test_momentum_gather_t1_products_host_logic(cpu_abi):
+def test_momentum_gather_t1_products_from_block_rule_host_logic(cpu_abi):
     """``pmb_gather_expand``: the T1 dressing products of a stored UEG block with ONE summed index
     (ccsd.py:322-419: "abid,dj->abij", "abcj,ci->abij", "iabc,cj->iabj", "iacb,cj->iajb") through
     the partner tables (one candidate orbital per (x0,x1,x2), ueg.py:395-404), against the dense
@@ -1252,7 +1252,7 @@ def test_momentum_gather_t1_products_host_logic(cpu_abi):
             assert calls["gather"] == n0 + 1, spec
             np.testing.assert_allclose(_n(got), np.einsum(spec, _n(A), _n(B)), rtol=0, atol=1e-13)
         # the tables hold exactly the non-zero structure of the block
-        tab = bk.geom_of(dV["abic"]).partner_tables(dV["abic"], 3)
+        tab = bk.partner_tables(dV["abic"], 3)
         assert tab["n_hit"] >= np.count_nonzero(_n(dV["abic"])) > 0
         # coefficient + accumulation into an existing tensor (a row of the dressed V_abij)
         R0 = rng.standard_normal((nv, nv, no, no))
@@ -1284,14 +1284,40 @@ def test_momentum_gather_t1_products_host_logic(cpu_abi):
         bk.set_gather(old)
 
 
-def test_momentum_groups_cover_every_nonzero_for_every_split():
+def test_blocked_companion_follows_in_place_edits(cpu_abi):
+    """V_iabc / V_aibc come with a never-stored twin for their products with tau; once a block is
+    edited in place the twin holds the old values and is not used: ``pair_with_tau`` computes with
+    the edited block."""
+    from pymes_b200 import backend as bk
+    from pymes_b200.model import ueg
+    from pymes_b200.solver import ccsd
+    m = ueg.UEG(14, 7, 7, 0.5)
+    m.init_single_basis(2.0)
+    m.gamma, m.k_cutoff = None, 1.0
+    no = 7
+    nv = m.n_orb - no
+    dV = m.eval_2b_blocks(no, ["iabc", "aibc"], [("only_non_hermi_2b", m.trunc), ("effect_2b", m.trunc)])
+    assert bk.blocked_companion(dV["iabc"]) is not None
+    dV["iabc"].mul_(2.0)
+    assert bk.blocked_companion(dV["iabc"]) is None
+    tau = _t(np.random.default_rng(13).standard_normal((nv, nv, no, no)))
+    W1, W2 = ccsd.pair_with_tau(dV["iabc"], dV["aibc"], tau, no)
+    np.testing.assert_allclose(_n(W1), np.einsum("kbcd,cdij->kbij", _n(dV["iabc"]), _n(tau)), rtol=0, atol=1e-13)
+    np.testing.assert_allclose(_n(W2), np.einsum("alcd,cdij->alij", _n(dV["aibc"]), _n(tau)), rtol=0, atol=1e-13)
+
+
+def test_momentum_groups_cover_every_nonzero_for_every_split(cpu_abi):
     """Every non-zero of the oracle-built TC-UEG V_pqrs (the reference's triple loop restated,
     oracle/ueg_oracle.py) lies inside the groups of ``momentum_groups`` -- for all six ways of
-    splitting (p,q,r,s) into two row and two entry axes and for random sub-blocks (what the geometry
-    tags of stored blocks and their narrowed row blocks rely on) -- and the partner tables of
-    ``pmb_gather_expand`` name exactly the non-zero's position for each of the four summed axes."""
+    splitting (p,q,r,s) into two row and two entry axes and for random sub-blocks (what the block
+    marks of stored blocks and their narrowed row blocks rely on) -- and the partner tables of
+    ``pmb_gather_expand`` name exactly the non-zero's position for each of the four summed axes.
+    The lists of ``pmb_blocked_contract`` built from the block's momentum rule hold the groups of a
+    stable sort of the linearised labels, each with its members in the same order, and the partner
+    tables equal the ones recomputed here from those labels."""
     import itertools
     from oracle import ueg_oracle as uo
+    from pymes_b200 import backend as bk
     from pymes_b200.model import ueg
     mo = uo.UEG(14, 1.0).init_single_basis(3.0)
     mo.k_cutoff, mo.gamma = 2.0, None
@@ -1301,6 +1327,8 @@ def test_momentum_groups_cover_every_nonzero_for_every_split():
     m.init_single_basis(3.0)
     assert m.n_orb == nP and np.array_equal(m.k_int(), mo.kint)
     k, imax = m.k_int(), m.imax
+    n = 2 * imax + 1
+    lin = (n * n * k[:, 0] + n * k[:, 1] + k[:, 2]).astype(np.int64)
     rng = np.random.default_rng(0)
     blocks = [((0,) * 4, (nP,) * 4)]
     for _ in range(4):
@@ -1323,13 +1351,46 @@ def test_momentum_groups_cover_every_nonzero_for_every_split():
             ents = nz[:, k_axes[0]] * ext[k_axes[1]] + nz[:, k_axes[1]]
             assert (row_gid[rows] >= 0).all() and (row_gid[rows] == ent_gid[ents]).all(), (lo, ext, m_axes)
             n_checked += len(nz)
+            # the groups of a stable sort of the labels, those of momentum_groups and those of the
+            # lists built from the rule: the same members in the same order
+            l = [ueg.SIGNS[ax] * lin[lo[ax]:lo[ax] + ext[ax]] for ax in range(4)]
+            row_key = np.add.outer(l[m_axes[0]], l[m_axes[1]]).reshape(-1)
+            ent_key = -np.add.outer(l[k_axes[0]], l[k_axes[1]]).reshape(-1)
+            keys = np.intersect1d(row_key, ent_key)
+            want = [(np.flatnonzero(row_key == g), np.flatnonzero(ent_key == g)) for g in keys]
+            L = bk.block_lists(ueg.momentum_rule(m, lo, ext), m_axes, k_axes)
+            L_rows = L["row_i0"] * ext[m_axes[1]] + L["row_i1"]
+            L_ents = L["ent_j0"] * ext[k_axes[1]] + L["ent_j1"]
+            got_mg = [(row_ord[r0:r0 + rn], ent_ord[e0:e0 + en]) for r0, rn, e0, en in zip(g_r0, g_rn, g_e0, g_en)]
+            assert len(got_mg) == len(want) == L["n_groups"]
+            for (wr, we), (gr, ge) in zip(want, got_mg):
+                assert np.array_equal(wr, gr) and np.array_equal(we, ge)
+            # every tile lies inside one group, and the tiles of a group cover its rows once
+            seen = {}
+            for m0, mn, e0, en in _n(L["tiles"]):
+                g = int(np.searchsorted(g_e0, e0))
+                assert g_e0[g] == e0 and g_en[g] == en and g_r0[g] <= m0 and m0 + mn <= g_r0[g] + g_rn[g]
+                seen.setdefault(g, []).extend(L_rows[m0:m0 + mn])
+            assert len(seen) == len(want)
+            for g, (wr, we) in enumerate(want):
+                assert sorted(seen[g]) == list(wr) and np.array_equal(L_ents[g_e0[g]:g_e0[g] + g_en[g]], we)
+            assert L["nnz"] == int(sum(len(wr) * len(we) for wr, we in want))
         # one candidate partner per triple, on every axis
-        n = 2 * imax + 1
-        lin = (n * n * k[:, 0] + n * k[:, 1] + k[:, 2]).astype(np.int64)
+        S = bk.tag_block(torch.from_numpy(np.ascontiguousarray(blk)), ueg.momentum_rule(m, lo, ext))
         for y in range(4):
             others = [ax for ax in range(4) if ax != y]
             l = [ueg.SIGNS[ax] * lin[lo[ax]:lo[ax] + ext[ax]] for ax in range(4)]
             want = -ueg.SIGNS[y] * (l[others[0]][nz[:, others[0]]] + l[others[1]][nz[:, others[1]]]
                                     + l[others[2]][nz[:, others[2]]])
             assert np.array_equal(ueg.SIGNS[y] * l[y][nz[:, y]], want), (lo, ext, y)     # raw l(k_y)
+            # the partner tables: for each triple of the other axes, the one y with l_y = want
+            grid = np.meshgrid(*[np.arange(ext[ax]) for ax in others], indexing="ij")
+            want = -ueg.SIGNS[y] * sum(l[ax][g] for ax, g in zip(others, grid))
+            hit = want[..., None] == (ueg.SIGNS[y] * l[y])[None, None, None, :]
+            idx = np.where(hit.any(axis=-1), hit.argmax(axis=-1), -1)
+            tab = bk.partner_tables(S, y)
+            assert np.array_equal(_n(tab["idx"]).reshape(idx.shape), idx) and tab["n_hit"] == int(hit.sum())
+            assert tab["ext"] == tuple(ext[ax] for ax in others)
+            val = np.take_along_axis(np.moveaxis(blk, y, -1), np.maximum(idx, 0)[..., None], -1)[..., 0]
+            assert np.array_equal(_n(tab["val"]).reshape(idx.shape), np.where(idx >= 0, val, 0.0))
     assert n_checked > 10000

@@ -82,7 +82,7 @@ def _tagged_t2(bk, m, no, nv, rng, dV):
     return T
 
 
-def test_rules_derivation_and_invalidation(abi):
+def test_rules_and_block_mark_derivation_and_invalidation(abi):
     from pymes_b200 import backend as bk
     from pymes_b200.solver import ccd
     m, no, nv, parts = _ueg14()
@@ -104,15 +104,15 @@ def test_rules_derivation_and_invalidation(abi):
                        ("alci,cblj->abij", Xp, bk.lincomb([1.0, -1.0], [T, Tt])),
                        ("kbic,ackj->abij", dV["iajb"], T), ("abkl,klij->abij", T, dV["klij"])]:
         assert bk.momentum_of(bk.contract(spec, A, B)) == rule, spec
-    # an in-place edit outside the backend drops the tag (and the geometry tag of a stored block)
+    # an in-place edit outside the backend drops the tag (and the block mark of a stored block)
     U = bk.copy(T)
     assert bk.momentum_of(U) == rule
     U.mul_(2.0)
     assert bk.momentum_of(U) is None
     W = bk.copy(dV["ijab"])
-    assert bk.geom_of(W) is not None
+    assert bk.block_rule(W) is not None
     W.add_(1.0)
-    assert bk.geom_of(W) is None and bk.momentum_of(W) is None
+    assert bk.block_rule(W) is None and bk.momentum_of(W) is None
     # accumulating a product with a different rule drops the tag of the output
     R = bk.copy(T)
     bk.contract_terms("abij", [(1.0, "acik", Tt, "cbkj", Xai)], out=R, beta=1.0)
